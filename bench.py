@@ -4,6 +4,7 @@ collective), with the HBM roofline of the step, the end-to-end number through th
 CPU oracle timed on the host cores as the reported baseline.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--envs-per-gpu E | --global-envs G] [--impl reference]
+                    [--dump-outputs DIR]
 
 One "step" = one msoc_step call over this rank's shard = two kernel launches (the streaming contact-free kernel over
 all envs, then one persistent contact kernel over the envs it declined, by work class).  Under torchrun (N > 1) every
@@ -11,6 +12,9 @@ rank owns a contiguous range of global env indices: E envs each by default (weak
 every GPU), or G / N with --global-envs G (strong scaling: BASELINE config 4 as written, 1 048 576 envs split over
 2/4/8 GPUs).  At N = 1 the line also carries BASELINE config 3 (65 536 envs, eager and as a replayed CUDA graph) and
 config 5 (PPO rollout with the MLP policy in the loop) as sub-records.
+
+--dump-outputs DIR writes what the last timed step returned on rank 0 (see dump_outputs) as DIR/<name>.npy.  The
+inputs are seeded, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -29,6 +33,7 @@ BYTES_PER_ENV_STEP = 2194  # SURVEY.md section 8(d): 940 B read + 1 254 B writte
 METRIC = "env_steps_per_sec"
 UNIT = "env-steps/s"
 DEFAULT_ENVS_PER_GPU = 1_048_576  # BASELINE config 4's total (1 Mi envs); working set >> 126 MB L2
+DUMP_ENVS = 32768  # envs sampled for --dump-outputs: 1 088 B each over the six files, 36 MB in all
 WORKLOAD = ("2v2 soccer, {n} envs per GPU ({g} in all), config.json defaults, i.i.d. random actions U(-1,1) (random "
             "windows of a pre-generated device buffer), auto-reset in full-random mode, shaped rewards, episodes "
             "staggered over all phases")
@@ -370,11 +375,25 @@ def config5_record(torch, _capi, cfg, dev, world_note="per GPU"):
             "env_steps_per_s": n * T * R / (ms * 1e-3), "ms_per_rollout_step": ms / (T * R), "episodes": st["episodes"]}
 
 
+def dump_outputs(torch, np, sim, offset: int, out_dir: str) -> None:
+    """What the last step returned (obs, reward, done, goal, and the step's score) for a fixed, seeded sample of
+    DUMP_ENVS envs, in env order, as float32 (the integer flags and counts are exact there), plus the global index of
+    every sampled env (float64)."""
+    n = sim.num_envs
+    idx = np.sort(np.random.default_rng(0).choice(n, size=min(n, DUMP_ENVS), replace=False))
+    sel = torch.from_numpy(idx).to(sim.device)
+    os.makedirs(out_dir, exist_ok=True)
+    for name in ("obs", "reward", "done", "goal", "score"):
+        out = getattr(sim, name).index_select(0, sel).to(torch.float32).cpu().numpy()
+        np.save(os.path.join(out_dir, f"{name}.npy"), out)
+    np.save(os.path.join(out_dir, "env_index.npy"), (idx + offset).astype(np.float64))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=1000)
-    ap.add_argument("--warmup", type=int, default=100)
+    ap.add_argument("--steps", type=int, default=None, help="timed steps (default 1000; --impl reference: 5)")
+    ap.add_argument("--warmup", type=int, default=None, help="warm-up steps (default 100; --impl reference: 1)")
     ap.add_argument("--envs-per-gpu", type=int, default=DEFAULT_ENVS_PER_GPU)
     ap.add_argument("--global-envs", type=int, default=0, help="strong scaling: this many envs split over the GPUs")
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
@@ -382,11 +401,18 @@ def main():
     ap.add_argument("--e2e-steps", type=int, default=10)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the config-3 / config-5 sub-records")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step returned as DIR/<name>.npy")
     args = ap.parse_args()
-    if args.impl == "reference":
-        if args.steps > 20:
-            args.steps = 5
-        args.warmup = min(args.warmup, 1)
+    ref = args.impl == "reference"
+    if args.steps is None:
+        args.steps = 5 if ref else 1000  # a reference bench step is a whole 1000-step episode of 1024 envs on the CPU
+    if args.warmup is None:
+        args.warmup = 1 if ref else 100
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if ref:
+        if args.dump_outputs:
+            ap.error("--dump-outputs applies to the GPU path (--impl ours)")
         run_reference(args)
         return
 
@@ -444,6 +470,8 @@ def main():
         dist.all_reduce(stats_t)  # the only collective: one 64-byte sum per rollout
     e1.record()
     torch.cuda.synchronize(dev)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(torch, np, sim, offset, args.dump_outputs)
     classes = sim.class_counts()  # work classes of the last timed step on this rank (instrumentation)
     if dist is not None:
         dist.barrier()

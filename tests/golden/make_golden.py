@@ -43,12 +43,13 @@ o2, r2, d2, g2 = ora.step(act2, auto_reset=False)
 states2 = ora.get_states()
 for s, s1 in zip(states2, states1):
     s["hist"] = [s1["hist"][1], P.pose_of(s)]
-out = {"act1": act1, "act2": act2, "rew1": r1, "rew2": r2, "done1": d1, "done2": d2, "goal1": g1, "goal2": g2,
-       "obs1": o1, "obs2": o2}
+out = {"act1": act1, "act2": act2, "rew1": r1, "rew2": r2, "done1": d1, "done2": d2, "goal1": g1, "goal2": g2}
 for name, st in (("s0", states0), ("s1", states1), ("s2", states2)):
     out.update(G.pack(st, name))
+# the observation a step returns is the one its state holds: stored once, as s1_obs / s2_obs
+assert np.array_equal(o1, out["s1_obs"]) and np.array_equal(o2, out["s2_obs"])
 path = os.path.join(HERE, "step_v2.npz")
-np.savez_compressed(path, **out)
+G.save(path, out)
 nc = sum(len(s["cache"]) for s in states1)
 print(f"wrote {path}: {N} envs, {int(np.abs(g1).sum())}+{int(np.abs(g2).sum())} goals, {nc} cached arbiters after step 1, "
       f"{os.path.getsize(path) / 1e3:.0f} kB")

@@ -2,6 +2,8 @@
 (tests/golden/make_golden.py) and tests/test_golden.py.  TEST INFRASTRUCTURE."""
 from __future__ import annotations
 
+import zipfile
+
 import numpy as np
 
 MAXC = 32
@@ -33,6 +35,14 @@ def pack(states: list, prefix: str) -> dict:
             out[f"{prefix}_hist_{k}"] = np.stack([np.stack([np.asarray(s["hist"][j][k], np.float64) for j in range(2)])
                                                   for s in states])
     return out
+
+
+def save(path: str, arrays: dict) -> None:
+    """np.savez with LZMA instead of deflate, which keeps step_v2.npz under 1 MB; np.load reads it like any .npz."""
+    with zipfile.ZipFile(path, "w", compression=zipfile.ZIP_LZMA) as zf:
+        for k, v in arrays.items():
+            with zf.open(f"{k}.npy", "w") as f:
+                np.lib.format.write_array(f, np.asanyarray(v), allow_pickle=False)
 
 
 def unpack(z, prefix: str) -> list:

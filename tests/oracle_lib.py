@@ -281,10 +281,6 @@ class OracleVec:
 
 
 def load_reference_config() -> dict:
-    """config.json defaults; reads the reference's file when it is present (this container),
-    and always checks it equals the restated DEFAULT_CONFIG above."""
-    p = "/root/reference/soccer_simulation/config.json"
-    if os.path.exists(p):
-        with open(p) as f:
-            return json.load(f)
-    return DEFAULT_CONFIG
+    """The shipped copy of the reference's soccer_simulation/config.json (marl_soccer_b200/config.json)."""
+    with open(os.path.join(ROOT, "marl_soccer_b200", "config.json")) as f:
+        return json.load(f)

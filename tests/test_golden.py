@@ -24,8 +24,8 @@ def test_oracle_reproduces_the_golden_vectors_bit_exactly(gold):
     ora = O.OracleVec(n, P.CONFIG, seed=0)
     ora.set_states(gold["s0"])
     for k, (act, obs, rew, done, goal, want) in enumerate((
-            (z["act1"], z["obs1"], z["rew1"], z["done1"], z["goal1"], gold["s1"]),
-            (z["act2"], z["obs2"], z["rew2"], z["done2"], z["goal2"], gold["s2"]))):
+            (z["act1"], z["s1_obs"], z["rew1"], z["done1"], z["goal1"], gold["s1"]),
+            (z["act2"], z["s2_obs"], z["rew2"], z["done2"], z["goal2"], gold["s2"]))):
         o, r, d, g = ora.step(act, auto_reset=False)
         assert np.array_equal(o, obs) and np.array_equal(r, rew) and np.array_equal(d, done) and np.array_equal(g, goal), k
         for i, (a, b) in enumerate(zip(ora.get_states(), want)):
@@ -55,8 +55,8 @@ def _check(sim_cls, gold):
     velocities and observation history included): each is an independent check against the file."""
     z, n = gold["z"], len(gold["s0"])
     for k, (first, act, obs, rew, done, goal, want) in enumerate((
-            (gold["s0"], z["act1"], z["obs1"], z["rew1"], z["done1"], z["goal1"], gold["s1"]),
-            (gold["s1"], z["act2"], z["obs2"], z["rew2"], z["done2"], z["goal2"], gold["s2"]))):
+            (gold["s0"], z["act1"], z["s1_obs"], z["rew1"], z["done1"], z["goal1"], gold["s1"]),
+            (gold["s1"], z["act2"], z["s2_obs"], z["rew2"], z["done2"], z["goal2"], gold["s2"]))):
         sim = sim_cls(n, P.CONFIG, seed=0)
         sim.set_states(np.arange(n), [P.oracle_to_dev_state(s) for s in first])
         o_d, r_d, d_d, g_d = sim.step(act, auto_reset=False)

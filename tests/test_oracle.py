@@ -15,7 +15,7 @@ DT = 1.0 / 60.0
 
 
 def test_reference_config_matches_restated_defaults():
-    assert O.load_reference_config() == CFG  # reads /root/reference/.../config.json when present
+    assert O.load_reference_config() == CFG
 
 
 def test_philox_known_answers():
