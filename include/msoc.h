@@ -200,6 +200,20 @@ int msoc_device_buffers(msoc_handle *h, msoc_buffers *out);
    per env 4 x 66 floats) for a list of envs; synchronous. */
 int msoc_get_obs_host(msoc_handle *h, const int64_t *h_idx, int64_t n, float *h_obs);
 
+/* RGB images of envs, drawn on the device (no counterpart in the reference's batched path; the picture is the one of
+   marl_soccer_b200/renderer.py scene(): field, lines, agents with their noses, ball).  Each image shows the state
+   msoc_get_state returns: after a step the state behind the newest observation frame, after an auto-reset the first
+   state of the new episode, after msoc_set_state the injected state.
+     d_out  (n, height, width, 3) uint8, HWC, images contiguous; 16-byte aligned; every byte is written once
+   Pixel (r, c) shows the point ((c + 0.5) 800 / width, (r + 0.5) 600 / height) of the 800 x 600 screen (y down), so
+   the two axes scale independently.  The handle's state is not changed, nothing is allocated and the host does not
+   wait: the call can be captured in a CUDA graph behind msoc_step. */
+/* RGB images (n, height, width, 3) uint8 of the envs d_idx[0..n) (NULL: envs 0..n-1), stream-ordered, capturable.
+   An out-of-range device index yields an all-zero image and reads/writes nothing else. 1 <= height, width <= 4096. */
+int msoc_render(msoc_handle *h, const int64_t *d_idx, int64_t n, int height, int width, uint8_t *d_out, void *stream);
+/* Same with host index list and host output; validates indices (MSOC_ERR_INVALID), synchronous. */
+int msoc_render_host(msoc_handle *h, const int64_t *h_idx, int64_t n, int height, int width, uint8_t *h_out);
+
 /* Statistics: d_out receives 8 doubles (msoc_stats layout) on the device, stream-ordered, ready to
    be all-reduced with NCCL; reset != 0 zeroes the accumulators afterwards. */
 int msoc_stats_device(msoc_handle *h, double *d_out, int reset, void *stream);

@@ -11,7 +11,8 @@ import sys
 PKG = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(PKG)
 SRC = os.path.join(PKG, "csrc", "msoc.cu")
-DEPS = [SRC, os.path.join(PKG, "csrc", "step_core.cuh"), os.path.join(ROOT, "include", "msoc.h")]
+DEPS = [SRC, os.path.join(PKG, "csrc", "step_core.cuh"), os.path.join(PKG, "csrc", "render_core.cuh"),
+        os.path.join(ROOT, "include", "msoc.h")]
 OUT = os.path.join(PKG, "libmsoc.so")
 OUT_CHECKED = os.path.join(PKG, "libmsoc_checked.so")  # same sources with -DMSOC_CHECKS: the kernels' own bounds checks
 

@@ -26,6 +26,7 @@
 
 #include "../../include/msoc.h"
 #include "step_core.cuh"
+#include "render_core.cuh"
 
 using namespace msoc;
 
@@ -729,6 +730,84 @@ __global__ void __launch_bounds__(PI_X * PI_Y) msoc_policy_inputs_kernel(const f
     }
 }
 
+/* ------------------------------------------------------------------------------------ render */
+/* RGB images of a list of envs (render_core.cuh).  The output is write-only: n H W 3 bytes against 96 bytes of record
+   per env.  A block takes a tile of the flat pixel stream (a multiple of 32 pixels, at most RENDER_MAX_SPAN images):
+   the scenes of the tile's images are set up once, in shared memory; then every thread colours 32-pixel segments, and
+   each warp stages its 32 consecutive segments (3 072 contiguous bytes) in shared memory and writes them with
+   coalesced 16-byte stores -- every output byte once, nothing read back. */
+struct RenderParams {
+    Arrays A;
+    const int *ctl;
+    const int64_t *idx; /* n env indices or null: envs 0..n-1 */
+    uint8_t *out;       /* 16-byte aligned */
+    int64_t total_px, tile_px, tiles;
+    RenderGeom G;
+};
+
+__global__ void __launch_bounds__(RENDER_BLOCK) msoc_render_kernel(const __grid_constant__ RenderParams P)
+{
+    __shared__ RenderScene s_scene[RENDER_MAX_SPAN];
+    __shared__ __align__(16) uint32_t s_stage[RENDER_BLOCK / 32][32 * RENDER_SEG_WORDS];
+    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+    const int step = P.ctl[CTL_STEP_FAST];
+    const int64_t hw = (int64_t)P.G.H * P.G.W;
+    uint32_t *stage = s_stage[warp];
+#pragma unroll 1
+    for (int64_t tile = blockIdx.x; tile < P.tiles; tile += gridDim.x) {
+        const int64_t g_begin = tile * P.tile_px;
+        const int64_t g_end = g_begin + P.tile_px < P.total_px ? g_begin + P.tile_px : P.total_px;
+        const int64_t i0 = g_begin / hw;
+        const int span = (int)((g_end - 1) / hw - i0 + 1);
+        __syncthreads(); /* the previous tile's scenes are no longer read */
+        for (int k = tid; k < span; k += RENDER_BLOCK) {
+            const int64_t e = P.idx != nullptr ? P.idx[i0 + k] : i0 + k;
+            const bool ok = e >= 0 && e < P.A.n;
+            MSOC_CHECK(P.idx != nullptr || ok, CHK_RENDER);
+            render_scene(P.G, ok ? render_record(P.A, step, e) : nullptr, s_scene[k]);
+        }
+        __syncthreads();
+        const int base_off = (int)(g_begin - i0 * hw); /* pixel offset of the tile in image i0 */
+#pragma unroll 1
+        for (int s = 0; s < RENDER_SEGS_PER_THREAD; s++) {
+            const int64_t warp_g0 = g_begin + (int64_t)(s * RENDER_BLOCK + warp * 32) * RENDER_SEG;
+            if (warp_g0 >= g_end) break; /* warp-uniform */
+            const int64_t g0 = warp_g0 + (int64_t)lane * RENDER_SEG;
+            uint32_t w[RENDER_SEG_WORDS];
+            if (g0 < g_end) {
+                const int o = base_off + (int)(g0 - g_begin);
+                const int img = o / (int)hw, rem = o - img * (int)hw;
+                const int row = rem / P.G.W, col = rem - row * P.G.W;
+                const int count = g_end - g0 < RENDER_SEG ? (int)(g_end - g0) : RENDER_SEG;
+                uint32_t wm, bm, rm, ym, zm;
+                render_segment_masks(P.G, s_scene, img, row, col, count, wm, bm, rm, ym, zm);
+                render_pack(wm, bm, rm, ym, zm, w);
+                uint4 *st4 = reinterpret_cast<uint4 *>(stage + lane * RENDER_SEG_WORDS);
+#pragma unroll
+                for (int i = 0; i < RENDER_SEG_WORDS / 4; i++) st4[i] = make_uint4(w[4 * i], w[4 * i + 1], w[4 * i + 2], w[4 * i + 3]);
+            }
+            __syncwarp();
+            /* the warp's bytes [warp_g0 * 3, +3072) clipped to the tile (the rest belongs to the next tile's block, and
+               the idle lanes staged nothing), as 16-byte stores, bytes at a ragged end */
+            const int64_t byte0 = warp_g0 * 3;
+            const int64_t valid = (g_end - warp_g0) * 3 < 32 * RENDER_SEG * 3 ? (g_end - warp_g0) * 3 : 32 * RENDER_SEG * 3;
+            const uint4 *src = reinterpret_cast<const uint4 *>(stage);
+#pragma unroll
+            for (int i = 0; i < RENDER_SEG_WORDS / 4; i++) {
+                const int off = (i * 32 + lane) * 16;
+                if (off + 16 <= valid) {
+                    MSOC_CHECK(byte0 + off + 16 <= P.total_px * 3, CHK_RENDER);
+                    __stcs(reinterpret_cast<uint4 *>(P.out + byte0 + off), src[i * 32 + lane]);
+                } else if (off < valid) {
+                    const uint8_t *sb = reinterpret_cast<const uint8_t *>(src + i * 32 + lane);
+                    for (int b = 0; b < valid - off; b++) P.out[byte0 + off + b] = sb[b];
+                }
+            }
+            __syncwarp();
+        }
+    }
+}
+
 /* ---------------------------------------------------------------------------------- C-ABI */
 extern "C" {
 
@@ -1144,6 +1223,65 @@ int msoc_get_obs_host(msoc_handle *h, const int64_t *h_idx, int64_t n, float *h_
     g_launches++;
     CUDA_TRY(cudaGetLastError());
     CUDA_TRY(cudaMemcpy(h_obs, d_o, ob, cudaMemcpyDeviceToHost));
+    return MSOC_OK;
+}
+
+static int check_render_args(const msoc_handle *h, int64_t n, int height, int width, const char *who)
+{
+    if (!h) return fail(MSOC_ERR_INVALID, who);
+    if (n < 0) return fail(MSOC_ERR_INVALID, "render: negative image count");
+    if (height < 1 || height > RENDER_MAX_SIDE || width < 1 || width > RENDER_MAX_SIDE)
+        return fail(MSOC_ERR_INVALID, "render: height and width must be in [1, 4096]");
+    return MSOC_OK;
+}
+
+static int launch_render(msoc_handle *h, const int64_t *d_idx, int64_t n, int height, int width, uint8_t *d_out, cudaStream_t st)
+{
+    RenderParams P;
+    P.A = h->A; P.ctl = h->d_ctl; P.idx = d_idx; P.out = d_out;
+    render_geom(height, width, P.G);
+    P.total_px = n * height * width;
+    P.tile_px = render_tile_px((int64_t)height * width);
+    P.tiles = (P.total_px + P.tile_px - 1) / P.tile_px;
+    const int64_t grid_cap = (int64_t)h->sm_count * 64; /* tiles beyond that are taken grid-stride */
+    msoc_render_kernel<<<(unsigned)(P.tiles < grid_cap ? P.tiles : grid_cap), RENDER_BLOCK, 0, st>>>(P);
+    g_launches++;
+    CUDA_TRY(cudaGetLastError());
+    return MSOC_OK;
+}
+
+int msoc_render(msoc_handle *h, const int64_t *d_idx, int64_t n, int height, int width, uint8_t *d_out, void *stream)
+{
+    int rc = check_render_args(h, n, height, width, "msoc_render: null handle");
+    if (rc != MSOC_OK || n == 0) return rc;
+    if (!d_out || ((uintptr_t)d_out & 15u) != 0u) return fail(MSOC_ERR_INVALID, "msoc_render: output must be a 16-byte aligned device pointer");
+    if (!d_idx && n > h->n) return fail(MSOC_ERR_INVALID, "msoc_render: more images than envs");
+    DeviceGuard guard(h->device);
+    return launch_render(h, d_idx, n, height, width, d_out, (cudaStream_t)stream);
+}
+
+int msoc_render_host(msoc_handle *h, const int64_t *h_idx, int64_t n, int height, int width, uint8_t *h_out)
+{
+    int rc = check_render_args(h, n, height, width, "msoc_render_host: null handle");
+    if (rc != MSOC_OK || n == 0) return rc;
+    if (!h_out) return fail(MSOC_ERR_INVALID, "msoc_render_host: null output");
+    if (h_idx) {
+        rc = check_idx(h, h_idx, n, "msoc_render_host: bad argument");
+        if (rc != MSOC_OK) return rc;
+    } else if (n > h->n) {
+        return fail(MSOC_ERR_INVALID, "msoc_render_host: more images than envs");
+    }
+    DeviceGuard guard(h->device);
+    const size_t ib = align_up((size_t)n * sizeof(int64_t)), ob = (size_t)n * height * width * 3;
+    rc = ensure_stage(h, ib + ob);
+    if (rc != MSOC_OK) return rc;
+    int64_t *d_idx = h_idx ? (int64_t *)h->d_stage : nullptr;
+    uint8_t *d_o = (uint8_t *)h->d_stage + ib;
+    CUDA_TRY(cudaDeviceSynchronize());
+    if (h_idx) CUDA_TRY(cudaMemcpy(d_idx, h_idx, (size_t)n * sizeof(int64_t), cudaMemcpyHostToDevice));
+    rc = launch_render(h, d_idx, n, height, width, d_o, nullptr);
+    if (rc != MSOC_OK) return rc;
+    CUDA_TRY(cudaMemcpy(h_out, d_o, ob, cudaMemcpyDeviceToHost));
     return MSOC_OK;
 }
 

@@ -117,6 +117,18 @@ class HostBufferSim:
         _capi.check(self._L.msoc_get_obs_host(self._h, idx.ctypes.data, 1, o.ctypes.data))
         return o[0]
 
+    def render(self, idx=None, height: int = 600, width: int = 800) -> np.ndarray:
+        """RGB images (n, height, width, 3) uint8 of the envs `idx` (None: all), drawn on the device and copied back
+        (msoc_render_host); an index out of range raises."""
+        if idx is None:
+            n, iptr, keep = self.n, None, None
+        else:
+            keep = np.ascontiguousarray(idx, dtype=np.int64).reshape(-1)
+            n, iptr = int(keep.size), keep.ctypes.data
+        out = np.empty((n, int(height), int(width), 3), np.uint8)
+        _capi.check(self._L.msoc_render_host(self._h, iptr, n, int(height), int(width), out.ctypes.data))
+        return out
+
     def counters(self):
         score = np.zeros((self.n, 2), np.int32)
         steps = np.zeros((self.n,), np.int32)

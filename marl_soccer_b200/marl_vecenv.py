@@ -121,6 +121,10 @@ class SyncMultiAgentVecEnv:
         truncs = np.repeat(done.astype(bool)[:, None], 4, axis=1)
         return obs, rewards, terms, truncs, LazyInfos(self._sim.score.copy(), goal.copy())
 
+    def render(self, idx=(0,), height: int = 600, width: int = 800) -> np.ndarray:
+        """RGB images (len(idx), height, width, 3) uint8 of the envs `idx`, drawn on the GPU (HostBufferSim.render)."""
+        return self._sim.render(idx, height, width)
+
     def _dict_to_array(self, data_dict):
         return np.array([data_dict[a] for a in self.possible_agents])
 
@@ -164,6 +168,10 @@ class TorchSoccerVecEnv:
         r = torch.zeros((self.num_envs, 4), dtype=torch.float32, device=self.sim.device)
         r[:, :2] = self.sim.reward
         return r
+
+    def render(self, idx=None, height: int = 600, width: int = 800, out=None):
+        """RGB images (n, height, width, 3) uint8 on the device: BatchedSoccerSim.render."""
+        return self.sim.render(idx, height, width, out)
 
     def infos(self) -> LazyInfos:
         return LazyInfos(self.sim.score.cpu().numpy(), self.sim.goal.cpu().numpy())

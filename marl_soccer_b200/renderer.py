@@ -1,8 +1,12 @@
-"""One-env render pull-back (SURVEY.md section 8f rank 4): `SoccerEnv.render()` copies ONE env's five poses to the
-host (msoc_get_state) and hands them to this module.  `scene(poses)` turns them into draw primitives in screen
-coordinates -- the y axis flipped like the reference's drawing code (soccer_simulation/renderer.py:30-42,
-game/entities.py:37-57,86-88) -- and `PygameRenderer` draws those primitives when pygame is installed.  The
-simulator itself never renders; nothing here touches the GPU."""
+"""The picture of an env.  `scene(poses)` turns the five poses into draw primitives in screen coordinates -- the y axis
+flipped like the reference's drawing code (soccer_simulation/renderer.py:30-42, game/entities.py:37-57,86-88) -- and is
+the definition of what an env looks like.
+
+Two paths draw it.  Batches of envs are rasterised on the GPU where they live: `BatchedSoccerSim.render()` /
+`TorchSoccerVecEnv.render()` (uint8 CUDA tensors) and `HostBufferSim.render()` / `SyncMultiAgentVecEnv.render()`
+(NumPy), all through msoc_render (csrc/render_core.cuh turns each primitive of `scene()` into an exact test on the
+pixel centre).  `SoccerEnv(render_mode="human").render()` copies ONE env's poses to the host (msoc_get_state) and
+`PygameRenderer` draws the primitives when pygame is installed; nothing in this module touches the GPU."""
 from __future__ import annotations
 
 import math

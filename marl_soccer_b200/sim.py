@@ -133,6 +133,38 @@ class BatchedSoccerSim:
         _capi.check(self._L.msoc_last_class_counts(self._h, C.byref(out), self._stream()))
         return {"light": out[0], "heavy": out[1], "pair": out[2], "multi": out[3]}
 
+    def render(self, idx=None, height: int = 600, width: int = 800, out: torch.Tensor | None = None) -> torch.Tensor:
+        """RGB images of envs drawn on the device (the picture of renderer.scene()): a uint8 CUDA tensor
+        (n, height, width, 3), written on the current stream.  Each image shows the state get_states() returns.
+
+        idx: None (all envs), a host sequence / ndarray of env indices (checked here: ValueError), or an int64 CUDA
+        tensor (not checked on the host: an out-of-range index gives an all-zero image).  out: an optional
+        preallocated contiguous uint8 tensor of that shape on the sim's device, so that the call allocates nothing
+        and can be captured in a CUDA graph."""
+        if idx is None:
+            n, dptr = self.num_envs, None
+        elif isinstance(idx, torch.Tensor) and idx.is_cuda:
+            if idx.dtype != torch.int64 or idx.device != self.device or idx.dim() != 1:
+                raise ValueError("a CUDA index tensor must be 1-D int64 on the sim's device")
+            idx = idx.contiguous()
+            n, dptr = int(idx.numel()), idx.data_ptr()
+        else:
+            host = np.asarray(idx.cpu() if isinstance(idx, torch.Tensor) else idx)
+            if host.ndim != 1 or (host.size and not np.issubdtype(host.dtype, np.integer)):
+                raise ValueError("idx must be a 1-D sequence of integer env indices")
+            host = host.astype(np.int64)
+            if host.size and (host.min() < 0 or host.max() >= self.num_envs):
+                raise ValueError(f"env index out of range [0, {self.num_envs})")
+            idx = torch.from_numpy(host).to(self.device)
+            n, dptr = int(host.size), idx.data_ptr()
+        shape = (n, int(height), int(width), 3)
+        if out is None:
+            out = torch.empty(shape, dtype=torch.uint8, device=self.device)
+        elif tuple(out.shape) != shape or out.dtype != torch.uint8 or out.device != self.device or not out.is_contiguous():
+            raise ValueError(f"out must be a contiguous uint8 tensor of shape {shape} on {self.device}")
+        _capi.check(self._L.msoc_render(self._h, dptr, n, int(height), int(width), out.data_ptr(), self._stream()))
+        return out
+
     def get_states(self, idx) -> list:
         idx = np.ascontiguousarray(idx, dtype=np.int64)
         arr = (_capi.MsocEnvState * len(idx))()
