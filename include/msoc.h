@@ -177,9 +177,27 @@ int msoc_reset_host(msoc_handle *h, const uint8_t *h_mask, int mode, int has_see
    score (N,2) i32 = info["score"] (game/game.py:415), steps (N) i32. Synchronous gather. */
 int msoc_read_counters(msoc_handle *h, int32_t *h_score /* N*2 */, int32_t *h_steps /* N */, void *stream);
 
-/* State injection / extraction for a list of local env indices (host arrays); synchronous. */
+/* State injection / extraction for a list of local env indices (host arrays); synchronous.  msoc_set_state wraps the
+   agent angles on the host in double precision.  Both run the kernels of msoc_save_states / msoc_load_states. */
 int msoc_get_state(msoc_handle *h, const int64_t *h_idx, int64_t n, msoc_env_state *h_out);
 int msoc_set_state(msoc_handle *h, const int64_t *h_idx, int64_t n, const msoc_env_state *h_in);
+
+/* Device-side checkpointing, branching and cloning of envs: msoc_env_state records in DEVICE memory, n x 808 bytes.
+   Records of the envs d_idx[0..n) (NULL: envs 0..n-1) as msoc_env_state, into device memory; stream-ordered,
+   no allocation, no host wait, capturable.  d_out 16-byte aligned.  An out-of-range device index gives an all-zero
+   record (hist_valid = 0).  The bytes equal what msoc_get_state returns for the same env. */
+int msoc_save_states(msoc_handle *h, const int64_t *d_idx, int64_t n, msoc_env_state *d_out, void *stream);
+/* Installs d_in[k] into env d_idx[k], with the semantics of msoc_set_state; out-of-range entries are skipped, duplicate
+   destinations are undefined.  The observation buffer is not written (as msoc_set_state).  The first call on a handle
+   may allocate the injection side array; if it is missing while `stream` is capturing, returns MSOC_ERR_INVALID.
+   Graphs of msoc_step / msoc_reset captured before that allocation do not see the side array: call msoc_load_states or
+   msoc_set_state once before capturing any graph on a handle whose states will be loaded.
+   d_in 16-byte aligned.  Agent angles (ang, hist_ang) are taken bit for bit when |a| <= 3.14159274101257324 (float(pi),
+   the threshold of msoc_set_state's host wrap); larger ones are wrapped into [-pi, pi] on the device in single
+   precision, which may differ in the last bit from the double-precision host wrap of msoc_set_state.
+   Both calls: n == 0 is a no-op; a null handle, n < 0, NULL d_idx with n > the env count and a null or misaligned state
+   pointer give MSOC_ERR_INVALID. */
+int msoc_load_states(msoc_handle *h, const int64_t *d_idx, int64_t n, const msoc_env_state *d_in, void *stream);
 
 /* Device pointers of the handle's INTERNAL I/O buffers (the ones the *_host entry points use), so that a
    device-resident caller can wrap them zero-copy (e.g. as torch tensors through
@@ -245,7 +263,7 @@ uint64_t msoc_launch_count(void);
 
 /* Debug aid: bit set of the kernels' own bounds / invariant checks that failed since the last call (list entries
    inside the stepped range, contact-pool and overflow slots, arbiter-cache counts, env indices of the observation
-   builder, the device-side step counter, non-NaN state).  Only the checked build (libmsoc_checked.so, compiled with
+   builder, the device-side step counter, non-NaN state, render and state save / load indices).  Only the checked build (libmsoc_checked.so, compiled with
    -DMSOC_CHECKS by marl_soccer_b200/build.py) evaluates them; the product build returns -1. */
 int msoc_debug_errors(void);
 

@@ -9,6 +9,8 @@ from __future__ import annotations
 import ctypes as C
 import os
 
+import numpy as np
+
 PKG_DIR = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("MSOC_LIB", os.path.join(PKG_DIR, "libmsoc.so"))  # MSOC_LIB: kernel A/B experiments
 
@@ -23,7 +25,7 @@ EXPORTS = (
     "msoc_step", "msoc_step_host", "msoc_reset_host", "msoc_read_counters", "msoc_get_state",
     "msoc_set_state", "msoc_get_obs_host", "msoc_step_host_frames", "msoc_stats_device", "msoc_stats_read",
     "msoc_launch_count", "msoc_device_buffers", "msoc_debug_errors", "msoc_last_class_counts", "msoc_policy_inputs",
-    "msoc_render", "msoc_render_host",
+    "msoc_render", "msoc_render_host", "msoc_save_states", "msoc_load_states",
 )
 
 
@@ -49,6 +51,44 @@ class MsocEnvState(C.Structure):
         ("hist_pos", C.c_float * 2 * 5 * 2), ("hist_vel", C.c_float * 2 * 4 * 2),
         ("hist_ang", C.c_float * 4 * 2), ("hist_angvel", C.c_float * 4 * 2),
     ]
+
+
+ENV_STATE_BYTES = 808
+assert C.sizeof(MsocEnvState) == ENV_STATE_BYTES
+# the same record as a NumPy structured dtype (offsets from the ctypes struct): a host snapshot is an array of these
+ENV_STATE_DTYPE = np.dtype(MsocEnvState)
+
+
+def _field_layout():
+    """name -> (byte offset, shape, torch dtype) of every msoc_env_state field."""
+    import torch
+    scalars = {C.c_float: torch.float32, C.c_int32: torch.int32, C.c_uint32: torch.uint32, C.c_uint64: torch.uint64}
+    out = {}
+    for name, ctype in MsocEnvState._fields_:
+        shape = []
+        while hasattr(ctype, "_length_"):  # c_float * 2 * 5 is an array of 5 arrays of 2
+            shape.append(ctype._length_)
+            ctype = ctype._type_
+        out[name] = (getattr(MsocEnvState, name).offset, tuple(shape), scalars[ctype])
+    return out
+
+
+def state_fields(t) -> dict:
+    """Named, writable typed views of a (n, 808) uint8 tensor of msoc_env_state records, on any device: e.g.
+    state_fields(t)["pos"] is (n, 5, 2) float32, ["seed"] (n,) uint64, ["cache_info"] (n, 32) uint32.  Writes through
+    the views land in `t`.  (torch has few arithmetic kernels for uint32 / uint64; view those as int32 / int64 for
+    arithmetic.)"""
+    if t.dim() != 2 or t.shape[1] != ENV_STATE_BYTES or t.dtype.itemsize != 1 or t.dtype.is_floating_point:
+        raise ValueError(f"expected a (n, {ENV_STATE_BYTES}) uint8 tensor, got {tuple(t.shape)} {t.dtype}")
+    if t.stride(1) != 1 or t.stride(0) % 8 != 0 or t.storage_offset() % 8 != 0:
+        raise ValueError("state_fields needs rows of 808 contiguous bytes at 8-byte aligned offsets")
+    n = t.shape[0]
+    views = {}
+    for name, (off, shape, dt) in _field_layout().items():
+        count = int(np.prod(shape)) if shape else 1
+        v = t[:, off:off + count * dt.itemsize].view(dt)
+        views[name] = v.view((n, *shape)) if shape else v.view(n)
+    return views
 
 
 class MsocStats(C.Structure):
@@ -119,6 +159,8 @@ def declare(L) -> None:
     L.msoc_policy_inputs.argtypes = [vp, i64, vp, vp, vp, vp, vp, vp]
     L.msoc_render.argtypes = [vp, vp, i64, C.c_int, C.c_int, vp, vp]
     L.msoc_render_host.argtypes = [vp, vp, i64, C.c_int, C.c_int, vp]
+    L.msoc_save_states.argtypes = [vp, vp, i64, vp, vp]
+    L.msoc_load_states.argtypes = [vp, vp, i64, vp, vp]
 
 
 def lib():

@@ -577,107 +577,283 @@ __global__ void __launch_bounds__(BLOCK) msoc_reset_kernel(const __grid_constant
     if (P.obs_out != nullptr && m != 0u) obs_tile(P.A, P.cfg, P.obs_out, nullptr, step, s_stage[warp], m, e, lane);
 }
 
-/* -------------------------------------------------------------------- state inject / extract */
-__device__ __forceinline__ void hist_to_record(const msoc_env_state &S, int k, float4 *r)
+/* ------------------------------------------------------------------- state save / load (msoc_env_state) */
+/* Records of a list of envs as msoc_env_state (include/msoc.h) in device memory, and back.  The state array is large and
+   touched once, so both kernels are built around it: a warp takes a group of eight consecutive entries (8 x 808 = 6 464
+   bytes, a 16-byte multiple), staged in shared memory in the layout of the array and moved between shared and global
+   memory as coalesced 16-byte accesses -- every sector of the array is read or written once and in full.  Four lanes
+   serve one env: lane q of the env reads / writes float4 q and q + 4 of each of its 128-byte records, so that every
+   warp access of a record covers whole sectors.  The bias block and the arbiter-cache entries are touched only when the
+   record's flags say they exist: an env without contacts costs its two records, score, seed and spawn count. */
+enum { CHK_STATES = CHK_RENDER + 1 }; /* staging slots, cache counts read from a record, the step counter */
+constexpr int STATE_ENVS = 8;                                 /* envs per warp group */
+constexpr int STATE_WORDS = (int)(sizeof(msoc_env_state) / 4); /* 202 */
+constexpr int STATE_GROUP_U4 = STATE_ENVS * STATE_WORDS / 4;  /* 404 */
+constexpr int STATE_BLOCK = 128;
+static_assert(sizeof(msoc_env_state) == 808 && (STATE_ENVS * sizeof(msoc_env_state)) % 16 == 0, "msoc_env_state layout");
+/* word offsets in msoc_env_state */
+enum : int {
+    SW_POS = offsetof(msoc_env_state, pos) / 4, SW_VEL = offsetof(msoc_env_state, vel) / 4,
+    SW_ANG = offsetof(msoc_env_state, ang) / 4, SW_ANGVEL = offsetof(msoc_env_state, angvel) / 4,
+    SW_VBIAS = offsetof(msoc_env_state, vbias) / 4, SW_RET = offsetof(msoc_env_state, ep_return) / 4,
+    SW_STEPS = offsetof(msoc_env_state, steps) / 4, SW_SCORE = offsetof(msoc_env_state, score) / 4,
+    SW_MODE = offsetof(msoc_env_state, mode) / 4, SW_SPAWN = offsetof(msoc_env_state, spawn_count) / 4,
+    SW_CCOUNT = offsetof(msoc_env_state, cache_count) / 4, SW_SEED = offsetof(msoc_env_state, seed) / 4,
+    SW_CINFO = offsetof(msoc_env_state, cache_info) / 4, SW_HVALID = offsetof(msoc_env_state, hist_valid) / 4,
+    SW_HPOS = offsetof(msoc_env_state, hist_pos) / 4, SW_HVEL = offsetof(msoc_env_state, hist_vel) / 4,
+    SW_HANG = offsetof(msoc_env_state, hist_ang) / 4, SW_HANGVEL = offsetof(msoc_env_state, hist_angvel) / 4,
+};
+/* the bias block (4 float4 per env in Arrays::bias: vbias of the five bodies, then wbias) is words SW_VBIAS.. in order */
+static_assert(offsetof(msoc_env_state, wbias) == offsetof(msoc_env_state, vbias) + 40 && offsetof(msoc_env_state, cache_jn) == offsetof(msoc_env_state, cache_info) + 128,
+              "msoc_env_state layout");
+
+struct StateParams {
+    Arrays A;
+    const int *ctl;
+    const int64_t *idx; /* n env indices or null: envs 0..n-1 */
+    int64_t n;
+    uint8_t *states;    /* n x 808 bytes, 16-byte aligned */
+};
+
+/* the group of entries [t0, t0 + count) between global and shared memory, 16-byte accesses (8 at an odd-count end) */
+__device__ __forceinline__ void group_store(uint8_t *g, const uint32_t *s, int count, int lane)
 {
-    Pose Q;
-    for (int i = 0; i < 5; i++) { Q.px[i] = S.hist_pos[k][i][0]; Q.py[i] = S.hist_pos[k][i][1]; }
-    for (int i = 0; i < 4; i++) { Q.vx[i] = S.hist_vel[k][i][0]; Q.vy[i] = S.hist_vel[k][i][1]; Q.ang[i] = S.hist_ang[k][i]; Q.w[i] = S.hist_angvel[k][i]; }
-    pose_pack(Q, 0.0f, 0.0f, r);
-}
-__device__ __forceinline__ void record_to_hist(const float4 *r, msoc_env_state &S, int k)
-{
-    Pose Q; pose_unpack(r, Q);
-    for (int i = 0; i < 5; i++) { S.hist_pos[k][i][0] = Q.px[i]; S.hist_pos[k][i][1] = Q.py[i]; }
-    for (int i = 0; i < 4; i++) { S.hist_vel[k][i][0] = Q.vx[i]; S.hist_vel[k][i][1] = Q.vy[i]; S.hist_ang[k][i] = Q.ang[i]; S.hist_angvel[k][i] = Q.w[i]; }
-}
-/* same pose?  (bit patterns of the 26 floats a frame is made of; the ball velocity in r[4].zw is not part of it) */
-__device__ __forceinline__ bool same_pose(const float4 *a, const float4 *b)
-{
-    bool same = true;
-    for (int i = 0; i < 7; i++) {
-        same = same && __float_as_uint(a[i].x) == __float_as_uint(b[i].x) && __float_as_uint(a[i].y) == __float_as_uint(b[i].y);
-        if (i != 4) same = same && __float_as_uint(a[i].z) == __float_as_uint(b[i].z) && __float_as_uint(a[i].w) == __float_as_uint(b[i].w);
+    const int valid = count * (int)sizeof(msoc_env_state);
+    const uint4 *s4 = reinterpret_cast<const uint4 *>(s);
+#pragma unroll
+    for (int i = 0; i < (STATE_GROUP_U4 + 31) / 32; i++) {
+        const int k = i * 32 + lane, off = k * 16;
+        if (off + 16 <= valid) reinterpret_cast<uint4 *>(g)[k] = s4[k];
+        else if (off < valid) reinterpret_cast<uint2 *>(g + off)[0] = reinterpret_cast<const uint2 *>(s4 + k)[0];
     }
+}
+__device__ __forceinline__ void group_load(uint32_t *s, const uint8_t *g, int count, int lane)
+{
+    const int valid = count * (int)sizeof(msoc_env_state);
+    uint4 *s4 = reinterpret_cast<uint4 *>(s);
+#pragma unroll
+    for (int i = 0; i < (STATE_GROUP_U4 + 31) / 32; i++) {
+        const int k = i * 32 + lane, off = k * 16;
+        if (off + 16 <= valid) s4[k] = __ldcs(reinterpret_cast<const uint4 *>(g) + k);
+        else if (off < valid) reinterpret_cast<uint2 *>(s4 + k)[0] = __ldcs(reinterpret_cast<const uint2 *>(g + off));
+    }
+}
+
+/* the state's float4 f of a record (store_env_record order) -> its words of msoc_env_state */
+__device__ __forceinline__ void put_state_f4(uint32_t *w, int f, float4 v)
+{
+    if (f < 5) {
+        w[SW_POS + 2 * f] = __float_as_uint(v.x); w[SW_POS + 2 * f + 1] = __float_as_uint(v.y);
+        w[SW_VEL + 2 * f] = __float_as_uint(v.z); w[SW_VEL + 2 * f + 1] = __float_as_uint(v.w);
+    } else if (f < 7) {
+        const int o = f == 5 ? SW_ANG : SW_ANGVEL;
+        w[o] = __float_as_uint(v.x); w[o + 1] = __float_as_uint(v.y); w[o + 2] = __float_as_uint(v.z); w[o + 3] = __float_as_uint(v.w);
+    } else {
+        const uint32_t flags = __float_as_uint(v.z);
+        w[SW_ANGVEL + 4] = __float_as_uint(v.x); w[SW_STEPS] = __float_as_uint(v.y); w[SW_RET] = __float_as_uint(v.w);
+        w[SW_MODE] = (flags & FLAG_MODE_MASK) >> FLAG_MODE_SHIFT; w[SW_CCOUNT] = flags & FLAG_CACHE_MASK;
+    }
+}
+/* float4 f < 7 of a record -> history pose k (what a frame is made of: the ball velocity r[4].zw is not part of it) */
+__device__ __forceinline__ void put_hist_f4(uint32_t *w, int k, int f, float4 v)
+{
+    if (f < 5) {
+        w[SW_HPOS + 10 * k + 2 * f] = __float_as_uint(v.x); w[SW_HPOS + 10 * k + 2 * f + 1] = __float_as_uint(v.y);
+        if (f < 4) { w[SW_HVEL + 8 * k + 2 * f] = __float_as_uint(v.z); w[SW_HVEL + 8 * k + 2 * f + 1] = __float_as_uint(v.w); }
+    } else {
+        const int o = (f == 5 ? SW_HANG : SW_HANGVEL) + 4 * k;
+        w[o] = __float_as_uint(v.x); w[o + 1] = __float_as_uint(v.y); w[o + 2] = __float_as_uint(v.z); w[o + 3] = __float_as_uint(v.w);
+    }
+}
+/* Angles: kept bit for bit when |a| <= float(pi) (the threshold of msoc_set_state's host wrap), otherwise wrapped with
+   the step's own range reduction -- which may differ in the last bit from the host's double-precision atan2 wrap. */
+__device__ __forceinline__ float state_angle(uint32_t bits)
+{
+    const float a = __uint_as_float(bits);
+    return (a > PI_F || a < -PI_F) ? wrap_angle(a) : a;
+}
+/* float4 f of the record of the state in w (store_env_record order; the flags word is the caller's) */
+__device__ __forceinline__ float4 get_state_f4(const uint32_t *w, int f, uint32_t flags)
+{
+    if (f < 5) return make_float4(__uint_as_float(w[SW_POS + 2 * f]), __uint_as_float(w[SW_POS + 2 * f + 1]),
+                                  __uint_as_float(w[SW_VEL + 2 * f]), __uint_as_float(w[SW_VEL + 2 * f + 1]));
+    if (f == 5) return make_float4(state_angle(w[SW_ANG]), state_angle(w[SW_ANG + 1]), state_angle(w[SW_ANG + 2]), state_angle(w[SW_ANG + 3]));
+    if (f == 6) return make_float4(__uint_as_float(w[SW_ANGVEL]), __uint_as_float(w[SW_ANGVEL + 1]), __uint_as_float(w[SW_ANGVEL + 2]), __uint_as_float(w[SW_ANGVEL + 3]));
+    return make_float4(__uint_as_float(w[SW_ANGVEL + 4]), __uint_as_float(w[SW_STEPS]), __uint_as_float(flags), __uint_as_float(w[SW_RET]));
+}
+/* float4 f < 7 of the record of history pose k (pose_pack order, ball velocity 0) */
+__device__ __forceinline__ float4 get_hist_f4(const uint32_t *w, int k, int f)
+{
+    if (f < 4) return make_float4(__uint_as_float(w[SW_HPOS + 10 * k + 2 * f]), __uint_as_float(w[SW_HPOS + 10 * k + 2 * f + 1]),
+                                  __uint_as_float(w[SW_HVEL + 8 * k + 2 * f]), __uint_as_float(w[SW_HVEL + 8 * k + 2 * f + 1]));
+    if (f == 4) return make_float4(__uint_as_float(w[SW_HPOS + 10 * k + 8]), __uint_as_float(w[SW_HPOS + 10 * k + 9]), 0.0f, 0.0f);
+    const int o = SW_HANG + 4 * k;
+    if (f == 5) return make_float4(state_angle(w[o]), state_angle(w[o + 1]), state_angle(w[o + 2]), state_angle(w[o + 3]));
+    const int p = SW_HANGVEL + 4 * k;
+    return make_float4(__uint_as_float(w[p]), __uint_as_float(w[p + 1]), __uint_as_float(w[p + 2]), __uint_as_float(w[p + 3]));
+}
+/* same bits in the part of float4 f that a frame is made of */
+__device__ __forceinline__ bool same_pose_f4(int f, float4 a, float4 b)
+{
+    bool same = __float_as_uint(a.x) == __float_as_uint(b.x) && __float_as_uint(a.y) == __float_as_uint(b.y);
+    if (f != 4) same = same && __float_as_uint(a.z) == __float_as_uint(b.z) && __float_as_uint(a.w) == __float_as_uint(b.w);
     return same;
 }
-
-__global__ void msoc_get_state_kernel(Arrays A, const int *ctl, const int64_t *idx, int64_t n, msoc_env_state *out)
+/* group index and validity of the env of lane group el */
+__device__ __forceinline__ int64_t state_env(const StateParams &P, int64_t t, bool &ok)
 {
-    const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (t >= n) return;
-    const int step = ctl[CTL_STEP_FAST];
-    const int64_t e = idx[t];
-    const float4 *rec = A.pose[buf_cur(step)] + e * POSE_F4;
-    const bool injected = (__float_as_uint(rec[7].z) & FLAG_INJECT) != 0u && A.inject != nullptr;
-    Env E;
-    load_env(A, injected ? A.inject + e * POSE_F4 : rec, e, E);
-    msoc_env_state S;
-    memset(&S, 0, sizeof S);
-    for (int i = 0; i < 5; i++) {
-        S.pos[i][0] = E.px[i]; S.pos[i][1] = E.py[i]; S.vel[i][0] = E.vx[i]; S.vel[i][1] = E.vy[i];
-        S.angvel[i] = E.w[i]; S.vbias[i][0] = E.vbx[i]; S.vbias[i][1] = E.vby[i];
-    }
-    for (int i = 0; i < 4; i++) { S.ang[i] = E.ang[i]; S.wbias[i] = E.wb[i]; }
-    S.ep_return = E.ep_return; S.steps = E.steps; S.score[0] = E.score_b; S.score[1] = E.score_r;
-    S.mode = (int)((E.flags & FLAG_MODE_MASK) >> FLAG_MODE_SHIFT);
-    S.spawn_count = A.spawn_count[e]; S.seed = A.seed[e];
-    const uint32_t cnt = E.flags & FLAG_CACHE_MASK;
-    S.cache_count = cnt;
-    for (uint32_t j = 0; j < cnt; j++) {
-        const uint32_t *c = A.cache[cache_half(step)] + cache_slot(e, (int)j);
-        S.cache_info[j] = c[0]; S.cache_jn[j] = __uint_as_float(c[1]); S.cache_jt[j] = __uint_as_float(c[2]);
-    }
-    S.hist_valid = 1u;
-    record_to_hist(A.pose[buf_prev(step)] + e * POSE_F4, S, 0);
-    record_to_hist(rec, S, 1);
-    out[t] = S;
+    const int64_t e = P.idx != nullptr ? P.idx[t] : t;
+    ok = e >= 0 && e < P.A.n;
+    MSOC_CHECK(P.idx != nullptr || ok, CHK_STATES);
+    return e;
 }
 
-__global__ void msoc_set_state_kernel(Arrays A, const int *ctl, const int64_t *idx, int64_t n, const msoc_env_state *in)
+/* Save: the bytes msoc_get_state returns -- the state (the injected record of a flagged env), the pose of the oldest
+   record as history 0 and the current record as history 1 (hist_valid = 1), cache entries, zeros after cache_count;
+   an out-of-range index gives an all-zero entry. */
+__global__ void __launch_bounds__(STATE_BLOCK) msoc_save_states_kernel(const __grid_constant__ StateParams P)
 {
-    const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (t >= n) return;
-    const int step = ctl[CTL_STEP_FAST];
-    const int64_t e = idx[t];
-    const msoc_env_state &S = in[t];
-    Env E;
-    for (int i = 0; i < 5; i++) {
-        E.px[i] = S.pos[i][0]; E.py[i] = S.pos[i][1]; E.vx[i] = S.vel[i][0]; E.vy[i] = S.vel[i][1];
-        E.w[i] = S.angvel[i]; E.vbx[i] = S.vbias[i][0]; E.vby[i] = S.vbias[i][1];
+    __shared__ __align__(16) uint32_t s_stage[STATE_BLOCK / 32][STATE_ENVS * STATE_WORDS];
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, el = lane >> 2, q = lane & 3;
+    const int64_t t0 = ((int64_t)blockIdx.x * (STATE_BLOCK / 32) + warp) * STATE_ENVS;
+    if (t0 >= P.n) return; /* warp-uniform */
+    const int count = P.n - t0 < STATE_ENVS ? (int)(P.n - t0) : STATE_ENVS;
+    uint32_t *stage = s_stage[warp];
+    const int step = P.ctl[CTL_STEP_FAST];
+    MSOC_CHECK(step >= 0 && step < 6, CHK_STATES);
+    bool ok = false;
+    const int64_t e = el < count ? state_env(P, t0 + el, ok) : 0;
+    const int f0 = q, f1 = q + 4;
+    float4 c0 = make_float4(0.0f, 0.0f, 0.0f, 0.0f), c1 = c0, p0 = c0, p1 = c0;
+    if (ok) {
+        const float4 *cur = P.A.pose[buf_cur(step)] + e * POSE_F4, *prev = P.A.pose[buf_prev(step)] + e * POSE_F4;
+        c0 = cur[f0]; c1 = cur[f1]; p0 = prev[f0];
+        if (f1 < 7) p1 = prev[f1];
     }
-    for (int i = 0; i < 4; i++) { E.ang[i] = S.ang[i]; E.wb[i] = S.wbias[i]; }
-    E.ep_return = S.ep_return; E.steps = S.steps; E.score_b = S.score[0]; E.score_r = S.score[1];
-    uint32_t cnt = S.cache_count > (uint32_t)MAX_CACHE ? (uint32_t)MAX_CACHE : S.cache_count;
-    E.flags = cnt | (((uint32_t)S.mode & 3u) << FLAG_MODE_SHIFT);
-    A.spawn_count[e] = S.spawn_count; A.seed[e] = S.seed;
-    for (uint32_t j = 0; j < cnt; j++) {
-        uint32_t *c = A.cache[cache_half(step)] + cache_slot(e, (int)j);
-        c[0] = S.cache_info[j]; c[1] = __float_as_uint(S.cache_jn[j]); c[2] = __float_as_uint(S.cache_jt[j]);
+    /* zero the staging area: out-of-range entries, the cache tail and the padding stay zero */
+    uint4 *stage4 = reinterpret_cast<uint4 *>(stage);
+#pragma unroll
+    for (int i = 0; i < (STATE_GROUP_U4 + 31) / 32; i++)
+        if (i * 32 + lane < STATE_GROUP_U4) stage4[i * 32 + lane] = make_uint4(0u, 0u, 0u, 0u);
+    /* lane 4 el + 3 holds float4 7 of the env's current record: flags */
+    const uint32_t cflags = __shfl_sync(0xffffffffu, __float_as_uint(c1.z), lane | 3);
+    float4 s0 = c0, s1 = c1;
+    if (ok && (cflags & FLAG_INJECT) != 0u && P.A.inject != nullptr) {
+        const float4 *inj = P.A.inject + e * POSE_F4;
+        s0 = inj[f0]; s1 = inj[f1];
     }
-    /* The observation history.  The frames already emitted stay what they were (the reference's deque is not touched by
-       a poke of the bodies): the current record keeps the pose behind the newest of them and the injected state goes to
-       Arrays::inject -- unless the two poses are the same bits.  With hist_valid the caller supplies both history poses
-       (checkpoint restore, parity injection). */
-    float4 *rec = A.pose[buf_cur(step)] + e * POSE_F4;
-    float4 newp[7], prev[7];
-    { Pose Q; pose_of(E, Q); pose_pack(Q, 0.0f, 0.0f, newp); }
-    if (S.hist_valid) {
-        float4 h0[7];
-        hist_to_record(S, 0, h0);
-        for (int i = 0; i < 7; i++) A.pose[buf_prev(step)][e * POSE_F4 + i] = h0[i];
-        hist_to_record(S, 1, prev);
+    const uint32_t flags = __shfl_sync(0xffffffffu, __float_as_uint(s1.z), lane | 3);
+    __syncwarp();
+    if (ok) {
+        uint32_t *w = stage + el * STATE_WORDS;
+        put_state_f4(w, f0, s0); put_state_f4(w, f1, s1);
+        put_hist_f4(w, 0, f0, p0); put_hist_f4(w, 1, f0, c0);
+        if (f1 < 7) { put_hist_f4(w, 0, f1, p1); put_hist_f4(w, 1, f1, c1); }
+        if (q == 0) {
+            const int2 sc = P.A.score[e];
+            w[SW_SCORE] = (uint32_t)sc.x; w[SW_SCORE + 1] = (uint32_t)sc.y;
+            w[SW_HVALID] = 1u;
+        } else if (q == 1) {
+            const uint64_t sd = P.A.seed[e];
+            w[SW_SEED] = (uint32_t)sd; w[SW_SEED + 1] = (uint32_t)(sd >> 32);
+            w[SW_SPAWN] = P.A.spawn_count[e];
+        }
+        if (flags & FLAG_HAS_BIAS) {
+            const float4 b = P.A.bias[4 * e + q];
+            w[SW_VBIAS + 4 * q] = __float_as_uint(b.x); w[SW_VBIAS + 4 * q + 1] = __float_as_uint(b.y);
+            if (q < 3) { w[SW_VBIAS + 4 * q + 2] = __float_as_uint(b.z); w[SW_VBIAS + 4 * q + 3] = __float_as_uint(b.w); }
+        }
+        /* cache entries j < count: 3 words each, contiguous per env (cache_slot), read as 16-byte chunks */
+        const uint32_t cnt = flags & FLAG_CACHE_MASK;
+        MSOC_CHECK(cnt <= (uint32_t)MAX_CACHE, CHK_STATES);
+        const int nw = 3 * (int)(cnt < (uint32_t)MAX_CACHE ? cnt : (uint32_t)MAX_CACHE);
+        const uint4 *c4 = reinterpret_cast<const uint4 *>(P.A.cache[cache_half(step)] + cache_slot(e, 0));
+        for (int c = q; 4 * c < nw; c += 4) {
+            const uint4 v = c4[c];
+            const uint32_t vv[4] = {v.x, v.y, v.z, v.w};
+#pragma unroll
+            for (int i = 0; i < 4; i++) {
+                const int word = 4 * c + i, j = word / 3;
+                MSOC_CHECK(word >= nw || j < MAX_CACHE, CHK_STATES);
+                if (word < nw) w[SW_CINFO + MAX_CACHE * (word - 3 * j) + j] = vv[i];
+            }
+        }
+    }
+    __syncwarp();
+    MSOC_CHECK(t0 + count <= P.n, CHK_STATES);
+    group_store(P.states + t0 * (int64_t)sizeof(msoc_env_state), stage, count, lane);
+}
+
+/* Load: what msoc_set_state did -- cache count clamped to MSOC_MAX_CACHE; hist_valid = 1 installs both history poses,
+   hist_valid = 0 keeps the emitted ones; a state whose pose differs from the newest emitted one goes to Arrays::inject
+   and its record is flagged FLAG_INJECT; the has-bias flag follows the bias values.  Out-of-range entries are skipped. */
+__global__ void __launch_bounds__(STATE_BLOCK) msoc_load_states_kernel(const __grid_constant__ StateParams P)
+{
+    __shared__ __align__(16) uint32_t s_stage[STATE_BLOCK / 32][STATE_ENVS * STATE_WORDS];
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, el = lane >> 2, q = lane & 3;
+    const int64_t t0 = ((int64_t)blockIdx.x * (STATE_BLOCK / 32) + warp) * STATE_ENVS;
+    if (t0 >= P.n) return; /* warp-uniform */
+    const int count = P.n - t0 < STATE_ENVS ? (int)(P.n - t0) : STATE_ENVS;
+    uint32_t *stage = s_stage[warp];
+    const int step = P.ctl[CTL_STEP_FAST];
+    MSOC_CHECK(step >= 0 && step < 6, CHK_STATES);
+    MSOC_CHECK(t0 + count <= P.n, CHK_STATES);
+    group_load(stage, P.states + t0 * (int64_t)sizeof(msoc_env_state), count, lane);
+    bool ok = false;
+    const int64_t e = el < count ? state_env(P, t0 + el, ok) : 0;
+    __syncwarp();
+    const uint32_t *w = stage + el * STATE_WORDS;
+    const int f0 = q, f1 = q + 4;
+    const uint32_t hist_valid = w[SW_HVALID];
+    /* the bias words of this lane's float4 of the bias block; any non-zero value in the env sets the has-bias flag */
+    float4 b = make_float4(__uint_as_float(w[SW_VBIAS + 4 * q]), __uint_as_float(w[SW_VBIAS + 4 * q + 1]), 0.0f, 0.0f);
+    if (q < 3) { b.z = __uint_as_float(w[SW_VBIAS + 4 * q + 2]); b.w = __uint_as_float(w[SW_VBIAS + 4 * q + 3]); }
+    const bool my_bias = b.x != 0.0f || b.y != 0.0f || b.z != 0.0f || b.w != 0.0f;
+    const uint32_t group = 0xfu << (lane & ~3);
+    const bool any_bias = (__ballot_sync(0xffffffffu, ok && my_bias) & group) != 0u;
+    const uint32_t ccount = w[SW_CCOUNT];
+    const uint32_t cnt = ccount > (uint32_t)MAX_CACHE ? (uint32_t)MAX_CACHE : ccount;
+    const uint32_t flags = cnt | ((w[SW_MODE] & 3u) << FLAG_MODE_SHIFT) | (any_bias ? FLAG_HAS_BIAS : 0u);
+    const float4 n0 = get_state_f4(w, f0, flags), n1 = get_state_f4(w, f1, flags);
+    float4 *rec = P.A.pose[buf_cur(step)] + (ok ? e : 0) * POSE_F4;
+    /* the pose behind the newest emitted frame: the caller's history pose 1, or what the current record holds */
+    float4 h0 = make_float4(0.0f, 0.0f, 0.0f, 0.0f), h1 = h0;
+    if (ok) {
+        if (hist_valid) { h0 = get_hist_f4(w, 1, f0); if (f1 < 7) h1 = get_hist_f4(w, 1, f1); }
+        else { h0 = rec[f0]; if (f1 < 7) h1 = rec[f1]; }
+    }
+    const bool my_same = same_pose_f4(f0, h0, n0) && (f1 >= 7 || same_pose_f4(f1, h1, n1));
+    const bool same = (__ballot_sync(0xffffffffu, !ok || my_same) & group) == group;
+    if (!ok) return; /* no warp-wide operation follows */
+    if (hist_valid) {
+        float4 *prev = P.A.pose[buf_prev(step)] + e * POSE_F4;
+        prev[f0] = get_hist_f4(w, 0, f0);
+        if (f1 < 7) prev[f1] = get_hist_f4(w, 0, f1);
+    }
+    if (any_bias) P.A.bias[4 * e + q] = b;
+    if (q == 0) P.A.score[e] = make_int2((int)w[SW_SCORE], (int)w[SW_SCORE + 1]);
+    else if (q == 1) { P.A.seed[e] = (uint64_t)w[SW_SEED] | ((uint64_t)w[SW_SEED + 1] << 32); P.A.spawn_count[e] = w[SW_SPAWN]; }
+    /* cache entries j < cnt of the current parity, as whole 16-byte chunks where the chunk lies inside them */
+    const int nw = 3 * (int)cnt;
+    uint32_t *cw = P.A.cache[cache_half(step)] + cache_slot(e, 0);
+    for (int c = q; 4 * c < nw; c += 4) {
+        uint32_t vv[4];
+#pragma unroll
+        for (int i = 0; i < 4; i++) { const int word = 4 * c + i, j = word / 3; vv[i] = word < nw ? w[SW_CINFO + MAX_CACHE * (word - 3 * j) + j] : 0u; }
+        if (4 * c + 4 <= nw) reinterpret_cast<uint4 *>(cw)[c] = make_uint4(vv[0], vv[1], vv[2], vv[3]);
+        else {
+#pragma unroll
+            for (int i = 0; i < 4; i++)
+                if (4 * c + i < nw) cw[4 * c + i] = vv[i];
+        }
+    }
+    if (same) {
+        rec[f0] = n0; rec[f1] = n1;
     } else {
-        for (int i = 0; i < 7; i++) prev[i] = rec[i];
-    }
-    store_env_bias(A, e, E);
-    A.score[e] = make_int2(E.score_b, E.score_r);
-    if (same_pose(prev, newp)) {
-        store_env_record(rec, E);
-    } else {
-        store_env_record(A.inject + e * POSE_F4, E);
-        for (int i = 0; i < 7; i++) rec[i] = prev[i];
-        rec[7] = make_float4(0.0f, __uint_as_float((uint32_t)E.steps), __uint_as_float(FLAG_INJECT), 0.0f);
+        float4 *inj = P.A.inject + e * POSE_F4;
+        inj[f0] = n0; inj[f1] = n1;
+        if (hist_valid) { rec[f0] = h0; if (f1 < 7) rec[f1] = h1; } /* otherwise the record already holds that pose */
+        if (f1 == 7) rec[7] = make_float4(0.0f, n1.y, __uint_as_float(FLAG_INJECT), 0.0f);
     }
 }
 
@@ -1146,6 +1322,33 @@ static int check_idx(const msoc_handle *h, const int64_t *idx, int64_t n, const 
     return MSOC_OK;
 }
 
+static int launch_states(msoc_handle *h, bool save, const int64_t *d_idx, int64_t n, void *d_states, cudaStream_t st)
+{
+    StateParams P;
+    P.A = h->A; P.ctl = h->d_ctl; P.idx = d_idx; P.n = n; P.states = (uint8_t *)d_states;
+    const int64_t envs_per_block = (STATE_BLOCK / 32) * STATE_ENVS;
+    const unsigned grid = (unsigned)((n + envs_per_block - 1) / envs_per_block);
+    if (save) msoc_save_states_kernel<<<grid, STATE_BLOCK, 0, st>>>(P);
+    else msoc_load_states_kernel<<<grid, STATE_BLOCK, 0, st>>>(P);
+    g_launches++;
+    CUDA_TRY(cudaGetLastError());
+    return MSOC_OK;
+}
+
+/* Arrays::inject: records of injected states whose pose differs from the newest emitted frame's */
+static int ensure_inject(msoc_handle *h, cudaStream_t st, const char *who)
+{
+    if (h->d_inject) return MSOC_OK;
+    cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
+    CUDA_TRY(cudaStreamIsCapturing(st, &cs));
+    if (cs != cudaStreamCaptureStatusNone)
+        return fail(MSOC_ERR_INVALID, "msoc_load_states: the first load on a handle allocates and cannot be captured; load once before capturing");
+    cudaError_t ce = cudaMalloc(&h->d_inject, (size_t)h->n * POSE_F4 * sizeof(float4));
+    if (ce != cudaSuccess) return fail(MSOC_ERR_ALLOC, who, ce);
+    h->A.inject = (float4 *)h->d_inject;
+    return MSOC_OK;
+}
+
 int msoc_get_state(msoc_handle *h, const int64_t *h_idx, int64_t n, msoc_env_state *h_out)
 {
     int rc = check_idx(h, h_idx, n, "msoc_get_state: bad argument");
@@ -1159,9 +1362,8 @@ int msoc_get_state(msoc_handle *h, const int64_t *h_idx, int64_t n, msoc_env_sta
     msoc_env_state *d_s = (msoc_env_state *)((char *)h->d_stage + ib);
     CUDA_TRY(cudaDeviceSynchronize());
     CUDA_TRY(cudaMemcpy(d_idx, h_idx, (size_t)n * sizeof(int64_t), cudaMemcpyHostToDevice));
-    msoc_get_state_kernel<<<(unsigned)((n + 127) / 128), 128>>>(h->A, h->d_ctl, d_idx, n, d_s);
-    g_launches++;
-    CUDA_TRY(cudaGetLastError());
+    rc = launch_states(h, true, d_idx, n, d_s, nullptr);
+    if (rc != MSOC_OK) return rc;
     CUDA_TRY(cudaMemcpy(h_out, d_s, sb, cudaMemcpyDeviceToHost));
     return MSOC_OK;
 }
@@ -1179,11 +1381,9 @@ int msoc_set_state(msoc_handle *h, const int64_t *h_idx, int64_t n, const msoc_e
     if (rc != MSOC_OK) return rc;
     if (!h_in) return fail(MSOC_ERR_INVALID, "msoc_set_state: null input");
     DeviceGuard guard(h->device);
-    if (!h->d_inject) { /* records of injected states whose pose differs from the newest emitted frame's */
-        cudaError_t ce = cudaMalloc(&h->d_inject, (size_t)h->n * POSE_F4 * sizeof(float4));
-        if (ce != cudaSuccess) return fail(MSOC_ERR_ALLOC, "msoc_set_state: cudaMalloc", ce);
-        h->A.inject = (float4 *)h->d_inject;
-    }
+    CUDA_TRY(cudaDeviceSynchronize());
+    rc = ensure_inject(h, nullptr, "msoc_set_state: cudaMalloc");
+    if (rc != MSOC_OK) return rc;
     const size_t ib = align_up((size_t)n * sizeof(int64_t)), sb = (size_t)n * sizeof(msoc_env_state);
     rc = ensure_stage(h, ib + sb);
     if (rc != MSOC_OK) return rc;
@@ -1196,14 +1396,40 @@ int msoc_set_state(msoc_handle *h, const int64_t *h_idx, int64_t n, const msoc_e
             S.ang[i] = wrap_host(S.ang[i]);
             for (int k = 0; k < 2; k++) S.hist_ang[k][i] = wrap_host(S.hist_ang[k][i]);
         }
-    CUDA_TRY(cudaDeviceSynchronize());
     CUDA_TRY(cudaMemcpy(d_idx, h_idx, (size_t)n * sizeof(int64_t), cudaMemcpyHostToDevice));
     CUDA_TRY(cudaMemcpy(d_s, tmp.data(), sb, cudaMemcpyHostToDevice));
-    msoc_set_state_kernel<<<(unsigned)((n + 127) / 128), 128>>>(h->A, h->d_ctl, d_idx, n, d_s);
-    g_launches++;
-    CUDA_TRY(cudaGetLastError());
+    rc = launch_states(h, false, d_idx, n, d_s, nullptr);
+    if (rc != MSOC_OK) return rc;
     CUDA_TRY(cudaDeviceSynchronize());
     return MSOC_OK;
+}
+
+static int check_states_args(const msoc_handle *h, const int64_t *d_idx, int64_t n, const void *d_states, const char *who)
+{
+    if (!h) return fail(MSOC_ERR_INVALID, who);
+    if (n < 0) return fail(MSOC_ERR_INVALID, "states: negative count");
+    if (n == 0) return MSOC_OK;
+    if (!d_states || ((uintptr_t)d_states & 15u) != 0u) return fail(MSOC_ERR_INVALID, "states: the state array must be a 16-byte aligned device pointer");
+    if (!d_idx && n > h->n) return fail(MSOC_ERR_INVALID, "states: more entries than envs");
+    return MSOC_OK;
+}
+
+int msoc_save_states(msoc_handle *h, const int64_t *d_idx, int64_t n, msoc_env_state *d_out, void *stream)
+{
+    int rc = check_states_args(h, d_idx, n, d_out, "msoc_save_states: null handle");
+    if (rc != MSOC_OK || n == 0) return rc;
+    DeviceGuard guard(h->device);
+    return launch_states(h, true, d_idx, n, d_out, (cudaStream_t)stream);
+}
+
+int msoc_load_states(msoc_handle *h, const int64_t *d_idx, int64_t n, const msoc_env_state *d_in, void *stream)
+{
+    int rc = check_states_args(h, d_idx, n, d_in, "msoc_load_states: null handle");
+    if (rc != MSOC_OK || n == 0) return rc;
+    DeviceGuard guard(h->device);
+    rc = ensure_inject(h, (cudaStream_t)stream, "msoc_load_states: cudaMalloc");
+    if (rc != MSOC_OK) return rc;
+    return launch_states(h, false, d_idx, n, (void *)d_in, (cudaStream_t)stream);
 }
 
 int msoc_get_obs_host(msoc_handle *h, const int64_t *h_idx, int64_t n, float *h_obs)

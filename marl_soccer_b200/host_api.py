@@ -105,6 +105,27 @@ class HostBufferSim:
         arr = (_capi.MsocEnvState * len(idx))(*states)
         _capi.check(self._L.msoc_set_state(self._h, idx.ctypes.data, len(idx), C.byref(arr)))
 
+    def save_states(self, idx) -> np.ndarray:
+        """States of the envs idx as an array of _capi.ENV_STATE_DTYPE (msoc_get_state straight into it).  The bytes are
+        the device format of BatchedSoccerSim.save_states:
+        torch.from_numpy(arr.view(np.uint8).reshape(n, 808)) moves a snapshot to the device."""
+        idx = np.ascontiguousarray(idx, dtype=np.int64).reshape(-1)
+        arr = np.zeros(idx.size, _capi.ENV_STATE_DTYPE)
+        if idx.size:
+            _capi.check(self._L.msoc_get_state(self._h, idx.ctypes.data, idx.size, arr.ctypes.data))
+        return arr
+
+    def load_states(self, idx, arr) -> None:
+        """Installs an array of _capi.ENV_STATE_DTYPE (or (n, 808) uint8) into the envs idx (msoc_set_state)."""
+        idx = np.ascontiguousarray(idx, dtype=np.int64).reshape(-1)
+        arr = np.ascontiguousarray(arr)
+        if arr.dtype != _capi.ENV_STATE_DTYPE:
+            arr = arr.view(np.uint8).reshape(-1).view(_capi.ENV_STATE_DTYPE)
+        if arr.size != idx.size:
+            raise ValueError(f"{idx.size} indices for {arr.size} states")
+        if idx.size:
+            _capi.check(self._L.msoc_set_state(self._h, idx.ctypes.data, idx.size, arr.ctypes.data))
+
     def get_state(self, i: int):
         return self.get_states([i])[0]
 

@@ -173,6 +173,13 @@ class TorchSoccerVecEnv:
         """RGB images (n, height, width, 3) uint8 on the device: BatchedSoccerSim.render."""
         return self.sim.render(idx, height, width, out)
 
+    def state_dict(self) -> dict:
+        """Env states, observation buffer and statistics: BatchedSoccerSim.state_dict."""
+        return self.sim.state_dict()
+
+    def load_state_dict(self, d: dict) -> None:
+        self.sim.load_state_dict(d)
+
     def infos(self) -> LazyInfos:
         return LazyInfos(self.sim.score.cpu().numpy(), self.sim.goal.cpu().numpy())
 

@@ -229,7 +229,8 @@ class GraphedRollout:
     msoc_step's two kernels -> storage) are captured once and replayed, so the ~30 launches per step cost no host
     time and the simulator is never waiting for Python.  The simulator's step counter lives in device memory, which
     is what makes a captured sequence of steps replayable (include/msoc.h).  Sampling uses torch's default CUDA
-    generator (graph-safe)."""
+    generator (graph-safe).  A sim whose states will be loaded (load_states, load_state_dict, clone_envs, set_states)
+    needs one such load before the graph is captured (include/msoc.h, msoc_load_states)."""
 
     def __init__(self, sim, agent: Agent, normalizer: RunningMeanStd, buf: RolloutBuffer, policy_dtype=None,
                  update_normalizer: bool = True):

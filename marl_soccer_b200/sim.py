@@ -79,6 +79,28 @@ class BatchedSoccerSim:
         self.goal = _view(bufs.goal, (n,), "|i1", d)
         self.score = _view(bufs.score, (n, 2), "<i4", d)
         self._stats = torch.zeros((8,), dtype=torch.float64, device=d)
+        self._stats_live = _view(bufs.stats, (8,), "<f8", d)  # the accumulators themselves (state_dict)
+
+    def _index(self, idx, unique: bool = False, n_all: int | None = None):
+        """(int64 CUDA tensor or None, count) of an env index argument: None (envs 0..n_all-1, default all), a host
+        sequence / ndarray / CPU tensor (checked: ValueError when out of range, or repeated with `unique`), or an int64
+        CUDA tensor on the sim's device (not checked)."""
+        if idx is None:
+            return None, self.num_envs if n_all is None else int(n_all)
+        if isinstance(idx, torch.Tensor) and idx.is_cuda:
+            if idx.dtype != torch.int64 or idx.device != self.device or idx.dim() != 1:
+                raise ValueError("a CUDA index tensor must be 1-D int64 on the sim's device")
+            idx = idx.contiguous()
+            return idx, int(idx.numel())
+        host = np.asarray(idx.cpu() if isinstance(idx, torch.Tensor) else idx)
+        if host.ndim != 1 or (host.size and not np.issubdtype(host.dtype, np.integer)):
+            raise ValueError("idx must be a 1-D sequence of integer env indices")
+        host = host.astype(np.int64)
+        if host.size and (host.min() < 0 or host.max() >= self.num_envs):
+            raise ValueError(f"env index out of range [0, {self.num_envs})")
+        if unique and np.unique(host).size != host.size:
+            raise ValueError("env indices to write must not repeat")
+        return torch.from_numpy(host).to(self.device), int(host.size)
 
     def close(self) -> None:
         if getattr(self, "_h", None):
@@ -141,22 +163,8 @@ class BatchedSoccerSim:
         tensor (not checked on the host: an out-of-range index gives an all-zero image).  out: an optional
         preallocated contiguous uint8 tensor of that shape on the sim's device, so that the call allocates nothing
         and can be captured in a CUDA graph."""
-        if idx is None:
-            n, dptr = self.num_envs, None
-        elif isinstance(idx, torch.Tensor) and idx.is_cuda:
-            if idx.dtype != torch.int64 or idx.device != self.device or idx.dim() != 1:
-                raise ValueError("a CUDA index tensor must be 1-D int64 on the sim's device")
-            idx = idx.contiguous()
-            n, dptr = int(idx.numel()), idx.data_ptr()
-        else:
-            host = np.asarray(idx.cpu() if isinstance(idx, torch.Tensor) else idx)
-            if host.ndim != 1 or (host.size and not np.issubdtype(host.dtype, np.integer)):
-                raise ValueError("idx must be a 1-D sequence of integer env indices")
-            host = host.astype(np.int64)
-            if host.size and (host.min() < 0 or host.max() >= self.num_envs):
-                raise ValueError(f"env index out of range [0, {self.num_envs})")
-            idx = torch.from_numpy(host).to(self.device)
-            n, dptr = int(host.size), idx.data_ptr()
+        idx, n = self._index(idx)
+        dptr = None if idx is None else idx.data_ptr()
         shape = (n, int(height), int(width), 3)
         if out is None:
             out = torch.empty(shape, dtype=torch.uint8, device=self.device)
@@ -164,6 +172,101 @@ class BatchedSoccerSim:
             raise ValueError(f"out must be a contiguous uint8 tensor of shape {shape} on {self.device}")
         _capi.check(self._L.msoc_render(self._h, dptr, n, int(height), int(width), out.data_ptr(), self._stream()))
         return out
+
+    def save_states(self, idx=None, out: torch.Tensor | None = None) -> torch.Tensor:
+        """msoc_env_state records of envs as a (n, 808) uint8 CUDA tensor, written on the current stream without a host
+        wait (the bytes of get_states; _capi.state_fields() gives named views).  idx as in render(): None (all envs), a
+        host sequence (checked: ValueError), or an int64 CUDA tensor (not checked: an out-of-range index gives an
+        all-zero record, whose hist_valid is 0).  out: an optional preallocated (n, 808) uint8 tensor on the sim's
+        device, so that the call allocates nothing and can be captured in a CUDA graph."""
+        idx, n = self._index(idx)
+        shape = (n, _capi.ENV_STATE_BYTES)
+        if out is not None and (tuple(out.shape) != shape or out.dtype != torch.uint8 or out.device != self.device):
+            raise ValueError(f"out must be a uint8 tensor of shape {shape} on {self.device}")
+        dst = out
+        if out is None or not out.is_contiguous() or out.data_ptr() % 16:
+            dst = torch.empty(shape, dtype=torch.uint8, device=self.device)
+        _capi.check(self._L.msoc_save_states(self._h, None if idx is None else idx.data_ptr(), n, dst.data_ptr(),
+                                             self._stream()))
+        if out is not None and dst is not out:  # a misaligned or strided `out` gets a copy
+            out.copy_(dst)
+        return out if out is not None else dst
+
+    def load_states(self, idx, states: torch.Tensor) -> None:
+        """Installs msoc_env_state records (n, 808) uint8 (save_states(), or built with _capi.state_fields()) into the
+        envs idx, on the current stream, with the semantics of set_states.  idx: None (envs 0..n-1), a host sequence
+        (checked: ValueError when out of range or repeated), or an int64 CUDA tensor (not checked: out-of-range entries
+        are skipped, repeated destinations are undefined).  The observation buffer is not written.  The first load on a
+        sim allocates a side array (the records of injected states), so it cannot be the first call inside a CUDA graph
+        capture.  A graph captured on this sim BEFORE that first load (or set_states) keeps stepping without the side
+        array: load (or set_states) once before capturing any graph on a sim whose states you will load."""
+        if not isinstance(states, torch.Tensor):
+            states = torch.from_numpy(np.ascontiguousarray(states).view(np.uint8).reshape(-1, _capi.ENV_STATE_BYTES))
+        if states.dim() != 2 or states.shape[1] != _capi.ENV_STATE_BYTES or states.dtype != torch.uint8:
+            raise ValueError(f"states must be a (n, {_capi.ENV_STATE_BYTES}) uint8 tensor")
+        idx, n = self._index(idx, unique=True, n_all=states.shape[0])
+        if n != states.shape[0]:
+            raise ValueError(f"{n} indices for {states.shape[0]} states")
+        if n > self.num_envs and idx is None:
+            raise ValueError(f"{n} states for {self.num_envs} envs")
+        if states.device != self.device or not states.is_contiguous() or states.data_ptr() % 16:
+            states = states.to(self.device).contiguous()
+            if states.data_ptr() % 16:
+                states = states.clone()
+        _capi.check(self._L.msoc_load_states(self._h, None if idx is None else idx.data_ptr(), n, states.data_ptr(),
+                                             self._stream()))
+
+    def clone_envs(self, src, dst) -> None:
+        """Env dst[k] becomes a copy of env src[k]: its state (save_states of src, then load_states) and its row of the
+        observation buffer.  src is snapshot before anything is written, so src and dst may overlap and src may
+        repeat; dst must not repeat.  Host index lists are checked (ValueError).  CUDA index tensors are not: a pair
+        with either index out of range is skipped, as load_states skips such entries, without a host wait."""
+        src_t, n = self._index(src)
+        dst_t, m = self._index(dst, unique=True)
+        if src is None or dst is None or n != m:
+            raise ValueError("src and dst must be index lists of the same length")
+        if n == 0:
+            return
+        N = self.num_envs
+        valid = (src_t >= 0) & (src_t < N) & (dst_t >= 0) & (dst_t < N)
+        snap = self.save_states(src_t)
+        # Observation rows, with torch indexing, which needs every index in range: a skipped pair repeats the copy of
+        # the first valid pair (the same bytes to the same row), or copies row 0 onto itself when no pair is valid.
+        j = torch.argmax(valid.to(torch.uint8)).view(1)
+        any_valid = valid.index_select(0, j)
+        src_r = torch.where(valid, src_t, torch.where(any_valid, src_t.index_select(0, j), 0))
+        dst_r = torch.where(valid, dst_t, torch.where(any_valid, dst_t.index_select(0, j), 0))
+        rows = self.obs.index_select(0, src_r)
+        self.load_states(torch.where(valid, dst_t, -1), snap)
+        self.obs.index_copy_(0, dst_r, rows)
+
+    STATE_FORMAT = "marl_soccer_b200.env_states/1"
+
+    def state_dict(self) -> dict:
+        """Everything needed to resume this sim exactly: every env's state (save_states()), the observation buffer (the
+        policy's next input, which the states do not determine), the 8 statistics accumulators, and what the states
+        are only valid for (config, env count, global env offset).  Tensors are copies on the sim's device.  The
+        outputs of the last step (reward, done, goal, score) are not part of it."""
+        return {"format": self.STATE_FORMAT, "num_envs": self.num_envs, "global_env_offset": self.global_env_offset,
+                "config": json.loads(json.dumps(self.config)), "states": self.save_states(),
+                "obs": self.obs.clone(), "stats": self._stats_live.clone()}
+
+    def load_state_dict(self, d: dict) -> None:
+        """Restores a state_dict() of a sim with the same env count, global env offset and config (ValueError
+        otherwise; load_states moves env states between differently shaped sims)."""
+        if d.get("format") != self.STATE_FORMAT:
+            raise ValueError(f"not a {self.STATE_FORMAT} state dict: format {d.get('format')!r}")
+        for key, mine in (("num_envs", self.num_envs), ("global_env_offset", self.global_env_offset),
+                          ("config", json.loads(json.dumps(self.config)))):
+            if d.get(key) != mine:
+                raise ValueError(f"state dict {key} {d.get(key)!r} does not match this sim's {mine!r}")
+        states, obs, stats = d["states"], d["obs"], d["stats"]
+        if tuple(states.shape) != (self.num_envs, _capi.ENV_STATE_BYTES) or tuple(obs.shape) != tuple(self.obs.shape) \
+                or tuple(stats.shape) != (8,):
+            raise ValueError("state dict tensors do not have this sim's shapes")
+        self.load_states(None, states)
+        self.obs.copy_(obs)
+        self._stats_live.copy_(stats)
 
     def get_states(self, idx) -> list:
         idx = np.ascontiguousarray(idx, dtype=np.int64)
