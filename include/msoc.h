@@ -251,6 +251,28 @@ int msoc_stats_read(msoc_handle *h, msoc_stats *h_out, int reset, void *stream);
 int msoc_policy_inputs(const float *d_obs, int64_t n_envs, const float *d_shift, const float *d_inv_std, void *d_x_out,
                        void *d_raw_out, double *d_moments, void *stream);
 
+/* The same pass over either team's rows, for a policy that plays red as if it were blue (self-play against frozen
+   snapshots; no counterpart in the reference, whose red agents play U(-1, 1)).  team 0 is msoc_policy_inputs: rows 0, 1
+   of every env.  team 1 reads rows 2, 3 (bytes 528..1055 of the env's 1056-byte block) and applies the mirror M below
+   to each of their three 22-float frames BEFORE the normalise, clip, bf16 and pad steps; d_raw_out and d_moments
+   receive the mirrored rows.  Output layout, NULL rules and the stream are those of msoc_policy_inputs (row 2e + a of
+   d_x_out = agent 2 + a of env e).  A team other than 0 or 1, a NULL d_obs / d_shift / d_inv_std / d_x_out or
+   n_envs <= 0 gives MSOC_ERR_INVALID.
+   The field is symmetric about x = 400 and red's frames are built from red's own side (mate a ^ 1, opponents 0 and 1,
+   own goal at x = 790), so M turns a red frame into the frame a blue agent sees on the mirrored field (x -> 800 - x,
+   theta -> pi - theta):
+     index                               feature                                mirrored
+     0, 1                                vx, vy / max_velocity                  -x, x
+     2                                   angle / pi                             x >= 0 ? 1 - x : -1 - x  (fp32; +0 and -0 -> 1)
+     3                                   omega / max_angular_velocity           -x
+     4, 7, 10, 13, 16, 19                unit-x to mate, opp 0, opp 1, ball,    -x
+                                         own goal, opp goal
+     5, 6, 8, 9, 11, 12, 14, 15, 17, 18, 20, 21   unit-y, distances             x
+   The negations are exact sign flips.  An action (a0, a1, a2) a mirrored policy returns (body-frame force x, y and
+   torque) is red's action (a0, -a1, -a2). */
+int msoc_team_inputs(const float *d_obs, int64_t n_envs, int team, const float *d_shift, const float *d_inv_std,
+                     void *d_x_out, void *d_raw_out, double *d_moments, void *stream);
+
 /* Work classes of the last step (instrumentation for tests and bench.py; no counterpart in the reference): how many envs
    the streaming kernel handed to the contact kernel as light (exactly one agent x wall candidate pair), heavy (the
    general path), pair (exactly one agent x agent / ball x agent pair, at most one wall pair beside it) and multi (several

@@ -25,7 +25,7 @@ EXPORTS = (
     "msoc_step", "msoc_step_host", "msoc_reset_host", "msoc_read_counters", "msoc_get_state",
     "msoc_set_state", "msoc_get_obs_host", "msoc_step_host_frames", "msoc_stats_device", "msoc_stats_read",
     "msoc_launch_count", "msoc_device_buffers", "msoc_debug_errors", "msoc_last_class_counts", "msoc_policy_inputs",
-    "msoc_render", "msoc_render_host", "msoc_save_states", "msoc_load_states",
+    "msoc_render", "msoc_render_host", "msoc_save_states", "msoc_load_states", "msoc_team_inputs",
 )
 
 
@@ -157,6 +157,7 @@ def declare(L) -> None:
     L.msoc_stats_read.argtypes = [vp, C.POINTER(MsocStats), C.c_int, vp]
     L.msoc_last_class_counts.argtypes = [vp, C.POINTER(C.c_int32 * 4), vp]
     L.msoc_policy_inputs.argtypes = [vp, i64, vp, vp, vp, vp, vp, vp]
+    L.msoc_team_inputs.argtypes = [vp, i64, C.c_int, vp, vp, vp, vp, vp, vp]
     L.msoc_render.argtypes = [vp, vp, i64, C.c_int, C.c_int, vp, vp]
     L.msoc_render_host.argtypes = [vp, vp, i64, C.c_int, C.c_int, vp]
     L.msoc_save_states.argtypes = [vp, vp, i64, vp, vp]

@@ -875,10 +875,14 @@ __global__ void msoc_init_kernel(Arrays A, uint64_t seed)
 }
 
 /* ------------------------------------------------------------------ rollout: policy inputs */
-/* One pass over the blue agents' observation rows (528 contiguous bytes per env): normalised + clipped bf16 policy input
+/* One pass over one team's observation rows (528 contiguous bytes per env): normalised + clipped bf16 policy input
    (padded rows), raw bf16 copy for the rollout buffer, per-feature sum / sum of squares for the running normaliser.
-   Thread (x, y): float2 x of the 132 floats of env y (+ 4 per iteration), so a thread always sees the same two features. */
+   Thread (x, y): float2 x of the 132 floats of env y (+ 4 per iteration), so a thread always sees the same two features.
+   TEAM 0 reads rows 0, 1 (blue) as they are.  TEAM 1 reads rows 2, 3 (red) and first mirrors them about x = 400
+   (include/msoc.h, msoc_team_inputs): a frame has an even length, so a thread's two features sit at the same even
+   offset g of every frame it sees, and its mirror is two fixed sign flips plus, at g = 2, the angle map. */
 constexpr int PI_X = 66, PI_Y = 4, PI_PAD = 72;
+template <int TEAM>
 __global__ void __launch_bounds__(PI_X * PI_Y) msoc_policy_inputs_kernel(const float *__restrict__ obs, int64_t n, const float *__restrict__ shift,
                                                                          const float *__restrict__ inv_std, __nv_bfloat162 *__restrict__ x_out,
                                                                          __nv_bfloat162 *__restrict__ raw_out, double *moments)
@@ -887,9 +891,17 @@ __global__ void __launch_bounds__(PI_X * PI_Y) msoc_policy_inputs_kernel(const f
     const int x = threadIdx.x, y = threadIdx.y;
     const int row = x >= 33 ? 1 : 0, f = 2 * x - 66 * row; /* features f, f + 1 of agent `row` */
     const float sh0 = shift[f], sh1 = shift[f + 1], is0 = inv_std[f], is1 = inv_std[f + 1];
+    /* the mirror of features g, g + 1 of a frame: negated are the x components 0, 3 (omega), 4, 7, 10, 13, 16, 19 */
+    const int g = f % FRAME;
+    const uint32_t neg0 = (g == 0 || g == 4 || g == 10 || g == 16) ? 0x80000000u : 0u;
+    const uint32_t neg1 = (g == 2 || g == 6 || g == 12 || g == 18) ? 0x80000000u : 0u;
     float s0 = 0.0f, s1 = 0.0f, q0 = 0.0f, q1 = 0.0f;
     for (int64_t e = (int64_t)blockIdx.x * PI_Y + y; e < n; e += (int64_t)gridDim.x * PI_Y) {
-        const float2 v = reinterpret_cast<const float2 *>(obs + e * (4 * OBS))[x];
+        float2 v = reinterpret_cast<const float2 *>(obs + e * (4 * OBS) + TEAM * (2 * OBS))[x];
+        if (TEAM == 1) {
+            v.x = g == 2 ? (v.x >= 0.0f ? 1.0f - v.x : -1.0f - v.x) : __uint_as_float(__float_as_uint(v.x) ^ neg0);
+            v.y = __uint_as_float(__float_as_uint(v.y) ^ neg1);
+        }
         const float a = fminf(fmaxf(fmaf(v.x, is0, sh0), -10.0f), 10.0f), b = fminf(fmaxf(fmaf(v.y, is1, sh1), -10.0f), 10.0f);
         x_out[((2 * e + row) * PI_PAD + f) >> 1] = __floats2bfloat162_rn(a, b);
         if (raw_out != nullptr) raw_out[(e * (2 * OBS) + 2 * x) >> 1] = __floats2bfloat162_rn(v.x, v.y);
@@ -982,6 +994,22 @@ __global__ void __launch_bounds__(RENDER_BLOCK) msoc_render_kernel(const __grid_
             __syncwarp();
         }
     }
+}
+
+/* msoc_policy_inputs / msoc_team_inputs after their argument checks */
+template <int TEAM>
+static int launch_policy_inputs(const float *d_obs, int64_t n_envs, const float *d_shift, const float *d_inv_std, void *d_x_out,
+                                void *d_raw_out, double *d_moments, void *stream)
+{
+    int dev = 0, sms = 0;
+    CUDA_TRY(cudaGetDevice(&dev));
+    CUDA_TRY(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+    const int64_t want = (n_envs + PI_Y - 1) / PI_Y, cap = (int64_t)sms * 7; /* 7 blocks of 264 threads per SM; a thread sums n / (4 * grid) rows in fp32 */
+    msoc_policy_inputs_kernel<TEAM><<<(unsigned)(want < cap ? want : cap), dim3(PI_X, PI_Y), 0, (cudaStream_t)stream>>>(
+        d_obs, n_envs, d_shift, d_inv_std, (__nv_bfloat162 *)d_x_out, (__nv_bfloat162 *)d_raw_out, d_moments);
+    g_launches++;
+    CUDA_TRY(cudaGetLastError());
+    return MSOC_OK;
 }
 
 /* ---------------------------------------------------------------------------------- C-ABI */
@@ -1533,15 +1561,16 @@ int msoc_policy_inputs(const float *d_obs, int64_t n_envs, const float *d_shift,
                        void *d_raw_out, double *d_moments, void *stream)
 {
     if (!d_obs || !d_shift || !d_inv_std || !d_x_out || n_envs <= 0) return fail(MSOC_ERR_INVALID, "msoc_policy_inputs: bad argument");
-    int dev = 0, sms = 0;
-    CUDA_TRY(cudaGetDevice(&dev));
-    CUDA_TRY(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-    const int64_t want = (n_envs + PI_Y - 1) / PI_Y, cap = (int64_t)sms * 7; /* 7 blocks of 264 threads per SM; a thread sums n / (4 * grid) rows in fp32 */
-    msoc_policy_inputs_kernel<<<(unsigned)(want < cap ? want : cap), dim3(PI_X, PI_Y), 0, (cudaStream_t)stream>>>(
-        d_obs, n_envs, d_shift, d_inv_std, (__nv_bfloat162 *)d_x_out, (__nv_bfloat162 *)d_raw_out, d_moments);
-    g_launches++;
-    CUDA_TRY(cudaGetLastError());
-    return MSOC_OK;
+    return launch_policy_inputs<0>(d_obs, n_envs, d_shift, d_inv_std, d_x_out, d_raw_out, d_moments, stream);
+}
+
+int msoc_team_inputs(const float *d_obs, int64_t n_envs, int team, const float *d_shift, const float *d_inv_std,
+                     void *d_x_out, void *d_raw_out, double *d_moments, void *stream)
+{
+    if (team != 0 && team != 1) return fail(MSOC_ERR_INVALID, "msoc_team_inputs: team must be 0 (blue) or 1 (red)");
+    if (!d_obs || !d_shift || !d_inv_std || !d_x_out || n_envs <= 0) return fail(MSOC_ERR_INVALID, "msoc_team_inputs: bad argument");
+    return team == 0 ? launch_policy_inputs<0>(d_obs, n_envs, d_shift, d_inv_std, d_x_out, d_raw_out, d_moments, stream)
+                     : launch_policy_inputs<1>(d_obs, n_envs, d_shift, d_inv_std, d_x_out, d_raw_out, d_moments, stream);
 }
 
 int msoc_last_class_counts(msoc_handle *h, int32_t h_out[4], void *stream)

@@ -119,27 +119,29 @@ class PackedPolicy:
       * biases ride in the GEMMs: every layer's output has 8 extra channels, the first of which is the constant 1
         (tanh of a pre-activation of 20), and the next layer's weight matrix carries its bias in that column -- a batched
         GEMM has no bias epilogue, and `baddbmm` materialises the broadcast bias with a strided copy [0.8 ms].
-    `refresh()` re-reads the agent's parameters (call it after every optimiser step)."""
+    `refresh()` re-reads the agent's parameters (call it after every optimiser step).
+    critic=False packs the actor alone (a stack of one net, for a policy whose value nobody reads: a frozen opponent);
+    the calls then return None for the value."""
 
     IN = 72
     PAD = 8       # extra channels per layer: [1, 0, 0, 0, 0, 0, 0, 0]
     ONE = 20.0    # tanh(20) == 1 in fp32 and bf16
 
-    def __init__(self, agent: Agent, dtype=torch.bfloat16):
-        self.agent, self.dtype = agent, dtype
+    def __init__(self, agent: Agent, dtype=torch.bfloat16, critic: bool = True):
+        self.agent, self.dtype, self.critic = agent, dtype, critic
         dev = agent.actor_logstd.device
-        P = self.PAD
-        self.w0 = torch.zeros((2 * (512 + P), self.IN), dtype=dtype, device=dev)
-        self.b0 = torch.zeros((2 * (512 + P),), dtype=dtype, device=dev)
+        P, S = self.PAD, 2 if critic else 1
+        self.w0 = torch.zeros((S * (512 + P), self.IN), dtype=dtype, device=dev)
+        self.b0 = torch.zeros((S * (512 + P),), dtype=dtype, device=dev)
         # hidden layers 512 -> 256 -> 128 -> 64 (each + PAD in and out), output layer 64 + PAD -> 8
-        self.w = [torch.zeros((2, o + P, i + P), dtype=dtype, device=dev) for o, i in ((256, 512), (128, 256), (64, 128))]
-        self.w.append(torch.zeros((2, 8, 64 + P), dtype=dtype, device=dev))
+        self.w = [torch.zeros((S, o + P, i + P), dtype=dtype, device=dev) for o, i in ((256, 512), (128, 256), (64, 128))]
+        self.w.append(torch.zeros((S, 8, 64 + P), dtype=dtype, device=dev))
         self.refresh()
 
     @torch.no_grad()
     def refresh(self) -> None:
         P = self.PAD
-        nets = (self.agent.actor_mean, self.agent.critic)
+        nets = (self.agent.actor_mean, self.agent.critic) if self.critic else (self.agent.actor_mean,)
         for k, net in enumerate(nets):
             base = (512 + P) * k
             self.w0[base:base + 512, :66].copy_(net[0].weight)
@@ -155,14 +157,15 @@ class PackedPolicy:
 
     @torch.no_grad()
     def __call__(self, x72: torch.Tensor):
-        """x72: (rows, 72) normalised observations in `dtype`, columns 66.. zero.  Returns (mean (rows, 3), value (rows, 1)) fp32."""
+        """x72: (rows, 72) normalised observations in `dtype`, columns 66.. zero.  Returns (mean (rows, 3), value (rows, 1)) fp32
+        (value None without the critic)."""
         rows = x72.shape[0]
         h = torch.addmm(self.b0, x72, self.w0.t()).tanh_()           # (rows, 2 * 520) = [actor 512 + 8 | critic 512 + 8]
-        h = h.view(rows, 2, 512 + self.PAD).transpose(0, 1)            # (2, rows, 520), strided: no copy
+        h = h.view(rows, self.w0.shape[0] // (512 + self.PAD), 512 + self.PAD).transpose(0, 1)  # (2, rows, 520), strided: no copy
         for j in range(3):
             h = torch.bmm(h, self.w[j].transpose(1, 2)).tanh_()
         out = torch.bmm(h, self.w[3].transpose(1, 2))                  # (2, rows, 8)
-        return out[0, :, :3].float(), out[1, :, :1].float()
+        return out[0, :, :3].float(), out[1, :, :1].float() if self.critic else None
 
     @torch.no_grad()
     def act(self, x72: torch.Tensor):
@@ -188,8 +191,10 @@ def _policy_step(agent, x, policy_dtype):
 @torch.no_grad()
 def collect_rollout(sim, agent: Agent, normalizer: RunningMeanStd, buf: RolloutBuffer, next_obs: torch.Tensor,
                     next_done: torch.Tensor, generator=None, update_normalizer: bool = True, policy_dtype=None,
-                    deterministic: bool = False):
-    """One rollout of `buf.obs.shape[0]` steps (marl-soccer.ipynb:366-431): blue = policy, red = U(-1, 1).
+                    deterministic: bool = False, opponent=None):
+    """One rollout of `buf.obs.shape[0]` steps (marl-soccer.ipynb:366-431): blue = policy, red = U(-1, 1), or red = the
+    frozen snapshots of `opponent` (selfplay.Opponent; it samples or plays its mean as it was built to, whatever
+    `deterministic` says).  Red's observations never reach the buffer or the normaliser.
     next_obs: (N, 2, 66) raw observations of the blue agents (may be a view of the simulator's observation buffer: it is
     consumed before the next step overwrites it); next_done: (N, 2).  Returns the updated pair (next_obs is a view of
     sim.obs).  policy_dtype: optional autocast dtype for the MLPs (e.g. torch.bfloat16); the simulator is always fp32.
@@ -211,7 +216,9 @@ def collect_rollout(sim, agent: Agent, normalizer: RunningMeanStd, buf: RolloutB
         buf.actions[t] = action.reshape(n, 2, 3)
         buf.logprobs[t] = logprob.reshape(n, 2)
         full[:, :2] = buf.actions[t]
-        if deterministic:
+        if opponent is not None:
+            opponent.act(sim)
+        elif deterministic:
             full[:, 2:] = 0.0
         else:
             full[:, 2:].uniform_(-1.0, 1.0, generator=generator)
@@ -230,11 +237,13 @@ class GraphedRollout:
     time and the simulator is never waiting for Python.  The simulator's step counter lives in device memory, which
     is what makes a captured sequence of steps replayable (include/msoc.h).  Sampling uses torch's default CUDA
     generator (graph-safe).  A sim whose states will be loaded (load_states, load_state_dict, clone_envs, set_states)
-    needs one such load before the graph is captured (include/msoc.h, msoc_load_states)."""
+    needs one such load before the graph is captured (include/msoc.h, msoc_load_states).
+    opponent: a selfplay.Opponent plays red inside the graph instead of U(-1, 1); Opponent.set() writes a new snapshot
+    into the buffers the graph reads, so the next replay plays it without a new capture."""
 
     def __init__(self, sim, agent: Agent, normalizer: RunningMeanStd, buf: RolloutBuffer, policy_dtype=None,
-                 update_normalizer: bool = True):
-        self.sim, self.agent, self.normalizer, self.buf = sim, agent, normalizer, buf
+                 update_normalizer: bool = True, opponent=None):
+        self.sim, self.agent, self.normalizer, self.buf, self.opponent = sim, agent, normalizer, buf, opponent
         self.policy_dtype, self.update_normalizer = policy_dtype, update_normalizer
         dev = sim.device
         self.mean32 = torch.zeros((66,), device=dev)
@@ -297,7 +306,10 @@ class GraphedRollout:
             buf.actions[t] = action.reshape(n, 2, 3)
             buf.logprobs[t] = logprob.reshape(n, 2)
             full[:, :2] = buf.actions[t]
-            full[:, 2:].uniform_(-1.0, 1.0)
+            if self.opponent is not None:
+                self.opponent.act(sim)
+            else:
+                full[:, 2:].uniform_(-1.0, 1.0)
             _obs, reward, done, _goal = sim.step(full, auto_reset=True)
             buf.rewards[t] = reward
             self.next_done.copy_(done.to(torch.float32)[:, None].expand(n, 2))
