@@ -159,6 +159,29 @@ int msoc_step(msoc_handle *h, const float *d_actions, float *d_obs_out,
               float *d_reward, uint8_t *d_done, int8_t *d_goal, int32_t *d_score, uint32_t flags,
               void *stream);
 
+/* msoc_step with a reward for both teams (self-play that trains on red's experience too; the reference has no red
+   reward).  Arguments, outputs, flags, stream semantics and graph capture are those of msoc_step, except:
+     d_reward  (N,4) f32, 16-byte aligned   columns 0, 1: blue's reward, bit for bit what msoc_step writes;
+                                            columns 2, 3: red's reward (the same for both red agents)
+   Red's reward is blue's reward on the field mirrored about x = 400 (msoc_team_inputs): in exact arithmetic, red's
+   reward of (S, actions) is blue's reward of M(S) with the mirrored actions.  Term by term, from the positions at the
+   start of the step and the step's displacement (before any soft reset), like blue's:
+     term            blue                                          red
+     proximity       ball_proximity_multiplier x decrease of the   the same for agents 2, 3
+                     distance of agents 0, 1 to the ball
+     ball to goal    move_ball_to_goal_multiplier x decrease of    the same to (10, 300)
+                     the ball's distance to (790, 300)
+     goals           +goal_scored_reward blue scores,              +goal_scored_reward red scores,
+                     -goal_conceded_penalty red scores             -goal_conceded_penalty blue scores
+     alive           -alive_penalty                                -alive_penalty
+     truncation      the step's reward becomes                     score_difference_multiplier x (red - blue)
+                     score_difference_multiplier x (blue - red)
+   Red's episode return is not kept by the handle (msoc_env_state.ep_return and msoc_stats stay blue's).  A misaligned
+   d_reward gives MSOC_ERR_INVALID, as do msoc_step's null arguments. */
+int msoc_step_teams(msoc_handle *h, const float *d_actions, float *d_obs_out,
+                    float *d_reward, uint8_t *d_done, int8_t *d_goal, int32_t *d_score, uint32_t flags,
+                    void *stream);
+
 /* Same call with HOST buffers (the NumPy drop-in path, marl_vecenv.py:62-68): copies actions
    H2D, steps, copies obs/reward/done/goal D2H and synchronises; NULL output pointers are skipped.  Large batches are
    cut into up to 8 chunks on two internal streams so that the H2D copy and the kernels of one chunk overlap the D2H

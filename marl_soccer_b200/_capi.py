@@ -26,6 +26,7 @@ EXPORTS = (
     "msoc_set_state", "msoc_get_obs_host", "msoc_step_host_frames", "msoc_stats_device", "msoc_stats_read",
     "msoc_launch_count", "msoc_device_buffers", "msoc_debug_errors", "msoc_last_class_counts", "msoc_policy_inputs",
     "msoc_render", "msoc_render_host", "msoc_save_states", "msoc_load_states", "msoc_team_inputs",
+    "msoc_step_teams",
 )
 
 
@@ -145,6 +146,7 @@ def declare(L) -> None:
     L.msoc_num_envs.restype = i64
     L.msoc_reset.argtypes = [vp, vp, C.c_int, C.c_int, u64, vp, vp]
     L.msoc_step.argtypes = [vp, vp, vp, vp, vp, vp, vp, u32, vp]
+    L.msoc_step_teams.argtypes = [vp, vp, vp, vp, vp, vp, vp, u32, vp]
     L.msoc_step_host.argtypes = [vp, vp, vp, vp, vp, vp, vp, u32, vp]
     L.msoc_step_host_frames.argtypes = [vp, vp, vp, vp, vp, vp, vp, u32, vp]
     L.msoc_reset_host.argtypes = [vp, vp, C.c_int, C.c_int, u64, vp, vp]

@@ -72,6 +72,7 @@ struct msoc_handle {
     SimCfg cfg;
     Arrays A;
     int sm_count, blocks_per_sm; /* persistent grid of the contact kernel */
+    int blocks_per_sm_teams;     /* the same for its TEAMS instance (msoc_step_teams) */
     int heavy_lanes_override; /* MSOC_HEAVY_LANES (experiments): 0 = choose by batch size */
     void *slab;
     /* internal I/O buffers of the host-buffer API */
@@ -108,7 +109,7 @@ struct StepParams {
     const float *actions; /* (N,4,3) */
     float *obs_out;       /* (N,4,66) */
     float *frames_out;    /* (N,4,22) or null */
-    float *reward;        /* (N,2) */
+    float *reward;        /* (N,2); (N,4), 16-byte aligned, in the TEAMS instances (msoc_step_teams) */
     uint8_t *done;        /* (N) */
     int8_t *goal;         /* (N) */
     int32_t *score;       /* (N,2) or null */
@@ -152,6 +153,7 @@ __device__ __forceinline__ int *step_ctl(const StepParams &P, int step) { return
 /* Loads env e (the record of buffer step % 3, or the injected record of a flagged env) and its actions, steps it.  On
    success (always, except for the contact-free mode, which declines envs that need the contact path) the per-env
    outputs and the new state are written; the observation follows in obs_tile once the whole warp has stored. */
+template <bool TEAMS>
 __device__ __forceinline__ bool step_one_env(const int MODE, const int ALLOWED, const StepParams &P, int step, int64_t e, Work &W, int &load, Tally &T)
 {
     float act[12];
@@ -172,8 +174,9 @@ __device__ __forceinline__ bool step_one_env(const int MODE, const int ALLOWED, 
     }
     load_env(P.A, rec, e, E);
     StepOut out;
-    if (!env_step(MODE, ALLOWED, E, act, P.cfg, P.A, cache_half(step), e, P.global_offset + (uint64_t)e, P.flags, W, out, load)) return false;
-    reinterpret_cast<float2 *>(P.reward)[e] = make_float2(out.reward, out.reward);
+    if (!env_step<TEAMS>(MODE, ALLOWED, E, act, P.cfg, P.A, cache_half(step), e, P.global_offset + (uint64_t)e, P.flags, W, out, load)) return false;
+    if (TEAMS) reinterpret_cast<float4 *>(P.reward)[e] = make_float4(out.reward, out.reward, out.reward_r, out.reward_r);
+    else reinterpret_cast<float2 *>(P.reward)[e] = make_float2(out.reward, out.reward);
     P.done[e] = out.done;
     P.goal[e] = out.goal;
     if (P.score != nullptr) reinterpret_cast<int2 *>(P.score)[e] = make_int2(out.score_b, out.score_r);
@@ -359,6 +362,8 @@ __device__ __forceinline__ void flush_tally(const Tally &T, double *stats, int l
     }
 }
 
+/* TEAMS (both step kernels): the step of msoc_step_teams, red's reward beside blue's (env_step) */
+template <bool TEAMS>
 __global__ void __launch_bounds__(FAST_BLOCK, MSOC_FAST_MIN_BLOCKS) msoc_step_fast_kernel(const __grid_constant__ StepParams P)
 {
     extern __shared__ __align__(16) float s_dyn[];
@@ -385,7 +390,7 @@ __global__ void __launch_bounds__(FAST_BLOCK, MSOC_FAST_MIN_BLOCKS) msoc_step_fa
     if (have) {
         /* the oldest of the three records the observation is rebuilt from is not needed by the step: start pulling it */
         asm volatile("prefetch.global.L2 [%0];" ::"l"(P.A.pose[buf_prev(step)] + my_env * POSE_F4));
-        ok = step_one_env(MODE_FAST, 1 << MODE_FAST, P, step, my_env, W, load, T);
+        ok = step_one_env<TEAMS>(MODE_FAST, 1 << MODE_FAST, P, step, my_env, W, load, T);
     }
     const uint32_t mask = __ballot_sync(0xffffffffu, ok);
     /* list slots of the declined envs, by work class: lanes 0..3 each fetch the base of one class (one atomic per warp and
@@ -439,7 +444,7 @@ constexpr size_t STEP_SMEM_BYTES = (size_t)(HEAVY_BLOCK / 32) * HEAVY_WARP_WORDS
    were measured to run one after the other on this part, not side by side): every warp pulls batches from one counter
    over the combined batch space [heavy | multi | pair | light], i.e. longest batches first, so that the few long
    latency-bound heavy batches start at once on their own warps while all the other warps stream through the rest. */
-template <int MODES>
+template <int MODES, bool TEAMS>
 __device__ __forceinline__ void contact_body(const StepParams &P, int *s_pool_count)
 {
     extern __shared__ __align__(16) float s_dyn[];
@@ -509,7 +514,7 @@ __device__ __forceinline__ void contact_body(const StepParams &P, int *s_pool_co
         __syncwarp();
         if (have) {
             asm volatile("prefetch.global.L2 [%0];" ::"l"(P.A.pose[buf_prev(step)] + my_env * POSE_F4));
-            ok = step_one_env(mode, MODES, P, step, my_env, W, load, T);
+            ok = step_one_env<TEAMS>(mode, MODES, P, step, my_env, W, load, T);
         }
         const uint32_t mask = __ballot_sync(0xffffffffu, ok);
         /* (obs_tile starts with a __syncwarp: the solver scratch of every lane is dead before it is reused) */
@@ -521,10 +526,11 @@ __device__ __forceinline__ void contact_body(const StepParams &P, int *s_pool_co
     flush_tally(T, P.stats, lane);
 }
 
+template <bool TEAMS>
 __global__ void __launch_bounds__(HEAVY_BLOCK, HEAVY_MIN_BLOCKS) msoc_step_contact_kernel(const __grid_constant__ StepParams P)
 {
     __shared__ int s_pool_count[HEAVY_BLOCK / 32];
-    contact_body<(1 << MODE_FULL) | (1 << MODE_LIGHT) | (1 << MODE_PAIR) | (1 << MODE_MULTI)>(P, s_pool_count);
+    contact_body<(1 << MODE_FULL) | (1 << MODE_LIGHT) | (1 << MODE_PAIR) | (1 << MODE_MULTI), TEAMS>(P, s_pool_count);
 }
 
 /* after a chunked host-buffer step (whose contact kernels do not): advances the step counter, sums the chunks' class counts */
@@ -1118,13 +1124,20 @@ int msoc_create(const msoc_config *cfg, int64_t n_envs, int device, uint64_t see
     h->d_ctl = (int *)(base + o_ctl);
     h->d_list = (int *)(base + o_list); h->d_list2 = (int *)(base + o_list2);
 
-    ce = cudaFuncSetAttribute(msoc_step_contact_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)STEP_SMEM_BYTES);
+    ce = cudaFuncSetAttribute(msoc_step_contact_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)STEP_SMEM_BYTES);
     if (ce == cudaSuccess)
-        ce = cudaFuncSetAttribute(msoc_step_fast_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)FAST_SMEM_BYTES);
+        ce = cudaFuncSetAttribute(msoc_step_fast_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)FAST_SMEM_BYTES);
+    if (ce == cudaSuccess)
+        ce = cudaFuncSetAttribute(msoc_step_contact_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)STEP_SMEM_BYTES);
+    if (ce == cudaSuccess)
+        ce = cudaFuncSetAttribute(msoc_step_fast_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)FAST_SMEM_BYTES);
     if (ce != cudaSuccess) return bail(MSOC_ERR_CUDA, "msoc_create: smem attribute", ce);
     cudaDeviceGetAttribute(&h->sm_count, cudaDevAttrMultiProcessorCount, device);
-    ce = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&h->blocks_per_sm, msoc_step_contact_kernel, HEAVY_BLOCK, STEP_SMEM_BYTES);
-    if (ce != cudaSuccess || h->blocks_per_sm < 1 || h->sm_count < 1) return bail(MSOC_ERR_CUDA, "msoc_create: occupancy query", ce);
+    ce = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&h->blocks_per_sm, msoc_step_contact_kernel<false>, HEAVY_BLOCK, STEP_SMEM_BYTES);
+    if (ce == cudaSuccess)
+        ce = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&h->blocks_per_sm_teams, msoc_step_contact_kernel<true>, HEAVY_BLOCK, STEP_SMEM_BYTES);
+    if (ce != cudaSuccess || h->blocks_per_sm < 1 || h->blocks_per_sm_teams < 1 || h->sm_count < 1)
+        return bail(MSOC_ERR_CUDA, "msoc_create: occupancy query", ce);
     if (ce == cudaSuccess) ce = cudaStreamCreateWithFlags(&h->pipe_stream, cudaStreamNonBlocking);
     if (ce == cudaSuccess) ce = cudaEventCreateWithFlags(&h->ev_pipe_fork, cudaEventDisableTiming);
     if (ce == cudaSuccess) ce = cudaEventCreateWithFlags(&h->ev_pipe_join, cudaEventDisableTiming);
@@ -1171,7 +1184,7 @@ int msoc_reset(msoc_handle *h, const uint8_t *d_mask, int mode, int has_seed, ui
 }
 
 /* the two launches of one step over the envs [e0, e1), both on `st` */
-static int launch_step(msoc_handle *h, StepParams &P, int64_t e0, int64_t e1, int chunk, cudaStream_t st)
+static int launch_step(msoc_handle *h, StepParams &P, int64_t e0, int64_t e1, int chunk, cudaStream_t st, bool teams = false)
 {
     P.e0 = e0; P.e1 = e1; P.chunk = chunk;
     const int64_t m = e1 - e0;
@@ -1188,10 +1201,10 @@ static int launch_step(msoc_handle *h, StepParams &P, int64_t e0, int64_t e1, in
     lf.dynamicSmemBytes = FAST_SMEM_BYTES;
     lf.stream = st;
     lf.attrs = at; lf.numAttrs = 1;
-    CUDA_TRY(cudaLaunchKernelEx(&lf, msoc_step_fast_kernel, P));
+    CUDA_TRY(cudaLaunchKernelEx(&lf, teams ? msoc_step_fast_kernel<true> : msoc_step_fast_kernel<false>, P));
     g_launches++;
     /* one persistent grid for all contact classes, right behind the streaming kernel */
-    const int64_t resident = (int64_t)h->sm_count * h->blocks_per_sm;
+    const int64_t resident = (int64_t)h->sm_count * (teams ? h->blocks_per_sm_teams : h->blocks_per_sm);
     const int64_t blocks_max = (m + HEAVY_BLOCK - 1) / HEAVY_BLOCK;
     cudaLaunchConfig_t lc = {};
     lc.gridDim = dim3((unsigned)(blocks_max < resident ? blocks_max : resident));
@@ -1199,7 +1212,7 @@ static int launch_step(msoc_handle *h, StepParams &P, int64_t e0, int64_t e1, in
     lc.dynamicSmemBytes = STEP_SMEM_BYTES;
     lc.stream = st;
     lc.attrs = at; lc.numAttrs = 1;
-    CUDA_TRY(cudaLaunchKernelEx(&lc, msoc_step_contact_kernel, P));
+    CUDA_TRY(cudaLaunchKernelEx(&lc, teams ? msoc_step_contact_kernel<true> : msoc_step_contact_kernel<false>, P));
     g_launches++;
     return MSOC_OK;
 }
@@ -1222,6 +1235,18 @@ int msoc_step(msoc_handle *h, const float *d_actions, float *d_obs_out, float *d
     StepParams P;
     fill_step_params(h, P, d_actions, d_obs_out, nullptr, d_reward, d_done, d_goal, d_score, flags);
     return launch_step(h, P, 0, h->n, -1, (cudaStream_t)stream);
+}
+
+int msoc_step_teams(msoc_handle *h, const float *d_actions, float *d_obs_out, float *d_reward,
+                    uint8_t *d_done, int8_t *d_goal, int32_t *d_score, uint32_t flags, void *stream)
+{
+    if (!h || !d_actions || !d_obs_out || !d_reward || !d_done || !d_goal)
+        return fail(MSOC_ERR_INVALID, "msoc_step_teams: null argument");
+    if ((uintptr_t)d_reward & 15u) return fail(MSOC_ERR_INVALID, "msoc_step_teams: d_reward must be 16-byte aligned");
+    DeviceGuard guard(h->device);
+    StepParams P;
+    fill_step_params(h, P, d_actions, d_obs_out, nullptr, d_reward, d_done, d_goal, d_score, flags);
+    return launch_step(h, P, 0, h->n, -1, (cudaStream_t)stream, true);
 }
 
 /* Host-buffer step: the envs are cut into chunks that alternate between two stream lanes, so that the H2D copy and the

@@ -943,6 +943,7 @@ MSOC_HD int popc32(uint32_t x)
 /* ------------------------------------------------------------------------------------------ step */
 struct StepOut {
     float reward;
+    float reward_r;       /* red's reward: set by the TEAMS instances of env_step only */
     uint8_t done;
     int8_t goal;
     bool fresh_episode;   /* auto-reset happened: obs = 3 copies of the new frame */
@@ -998,6 +999,20 @@ enum { IF_NX, IF_NY, IF_RN1, IF_RT1, IF_RN2, IF_RT2, IF_NM, IF_TM, IF_BIAS, IF_B
 enum { IF_U = IF_RN1 }; /* a static x body contact has no first arm: its slot carries the friction coefficient there */
 constexpr int ISL_SLOTS = 4;
 
+/* Shaping term of one distance (game/game.py:338,345): |d| - |d + l|, the decrease of the distance d over the step
+   displacement l, as the difference of squares over the sum of the two distances (no cancellation); 0 if both are 0. */
+MSOC_HD float distance_drop(float dx, float dy, float lx, float ly)
+{
+    const float dp = sqrtf(dx * dx + dy * dy);
+    const float nx_ = dx + lx, ny_ = dy + ly;
+    const float dc = sqrtf(nx_ * nx_ + ny_ * ny_);
+    const float den = dp + dc;
+    return den > 0.0f ? -(2.0f * (dx * lx + dy * ly) + (lx * lx + ly * ly)) / den : 0.0f;
+}
+
+/* TEAMS: red's reward too (out.reward_r), blue's reward on the field mirrored about x = 400 (include/msoc.h,
+   msoc_step_teams).  The TEAMS = false instances are the blue-only step, instruction for instruction. */
+template <bool TEAMS = false>
 MSOC_HD bool env_step(const int MODE, const int ALLOWED, Env &E, const float *act, const SimCfg &c, const Arrays &A, int cur, int64_t e,
                       uint64_t gidx, uint32_t step_flags, Work &W, StepOut &out, int &load)
 {
@@ -1039,6 +1054,10 @@ MSOC_HD bool env_step(const int MODE, const int ALLOWED, Env &E, const float *ac
     const float d0x = E.px[0] - E.px[4], d0y = E.py[0] - E.py[4];
     const float d1x = E.px[1] - E.px[4], d1y = E.py[1] - E.py[4];
     const float dgx = E.px[4] - FIELD_R, dgy = E.py[4] - 300.0f;
+    /* red's: agents 2, 3 to the ball, the ball to red's target (FIELD_L, 300) (its y offset is dgy) */
+    const float d2x = TEAMS ? E.px[2] - E.px[4] : 0.0f, d2y = TEAMS ? E.py[2] - E.py[4] : 0.0f;
+    const float d3x = TEAMS ? E.px[3] - E.px[4] : 0.0f, d3y = TEAMS ? E.py[3] - E.py[4] : 0.0f;
+    const float dhx = TEAMS ? E.px[4] - FIELD_L : 0.0f;
     E.steps += 1;
 
     /* ---- cpBodyUpdatePosition: p += (v + v_bias) dt, a += (w + w_bias) dt, bias cleared */
@@ -1155,7 +1174,7 @@ MSOC_HD bool env_step(const int MODE, const int ALLOWED, Env &E, const float *ac
 
     /* ---- shaping rewards (game/game.py:324-349) from the step displacement; only positions enter, so
        they are final here and their inputs need not stay live across the contact path */
-    float r = 0.0f;
+    float r = 0.0f, r_red = 0.0f;
     {
         const float ibx = incx[4], iby = incy[4];
         if (c.prox_mult != 0.0f) {
@@ -1186,6 +1205,11 @@ MSOC_HD bool env_step(const int MODE, const int ALLOWED, Env &E, const float *ac
             float imp = 0.0f;
             if (den > 0.0f) imp = -(2.0f * (dgx * ibx + dgy * iby) + (ibx * ibx + iby * iby)) / den;
             r += imp * c.move_mult;
+        }
+        if (TEAMS) { /* the same terms for red, in the same order */
+            if (c.prox_mult != 0.0f)
+                r_red += c.prox_mult * (distance_drop(d2x, d2y, incx[2] - ibx, incy[2] - iby) + distance_drop(d3x, d3y, incx[3] - ibx, incy[3] - iby));
+            r_red += distance_drop(dhx, dgy, ibx, iby) * c.move_mult;
         }
     }
 
@@ -1852,6 +1876,11 @@ MSOC_HD bool env_step(const int MODE, const int ALLOWED, Env &E, const float *ac
     if (goal > 0) r += c.goal_reward;
     if (goal < 0) r -= c.conceded_penalty;
     r -= c.alive_penalty;
+    if (TEAMS) {
+        if (goal < 0) r_red += c.goal_reward;
+        if (goal > 0) r_red -= c.conceded_penalty;
+        r_red -= c.alive_penalty;
+    }
 
     /* ---- soft reset on goal (game/game.py:421-422, :120-127): positions re-spawned in the current
        mode, velocities zeroed, agent angles 0/pi; ball angular velocity, biases, counters kept */
@@ -1871,9 +1900,10 @@ MSOC_HD bool env_step(const int MODE, const int ALLOWED, Env &E, const float *ac
     if (c.max_steps > 0 && E.steps >= c.max_steps) {
         done = true;
         r = c.score_diff_mult * (float)(E.score_b - E.score_r);
+        if (TEAMS) r_red = c.score_diff_mult * (float)(E.score_r - E.score_b);
     }
     E.ep_return += r;
-    out.reward = r; out.done = done ? 1 : 0; out.goal = (int8_t)goal;
+    out.reward = r; out.reward_r = r_red; out.done = done ? 1 : 0; out.goal = (int8_t)goal;
     out.fresh_episode = false; out.finished_return = 0.0f; out.score_dirty = goal != 0;
     out.n_contacts = n_contacts; out.overflow = overflow;
     out.score_b = E.score_b; out.score_r = E.score_r;

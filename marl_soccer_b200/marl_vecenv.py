@@ -159,8 +159,9 @@ class TorchSoccerVecEnv:
         mode = _capi.MODE_FIXED if use_fixed else _capi.MODE_FULL_RANDOM if use_full else _capi.MODE_RANDOM
         return self.sim.reset(mode, seed=seed)
 
-    def step(self, actions):
-        obs, rew, done, goal = self.sim.step(actions, auto_reset=True)
+    def step(self, actions, team_rewards: bool = False):
+        """team_rewards: rewards (N,4) f32 with red's own reward in columns 2, 3 (BatchedSoccerSim.step)."""
+        obs, rew, done, goal = self.sim.step(actions, auto_reset=True, team_rewards=team_rewards)
         return obs, rew, done.bool(), goal
 
     def rewards4(self):

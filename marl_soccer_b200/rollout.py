@@ -95,17 +95,51 @@ class RunningMeanStd:
         return torch.clamp((x - self.mean.float()) / (self.std.float() + 1e-8), -10.0, 10.0)
 
 
-class RolloutBuffer:
-    """(T, N, 2, ...) storage of one rollout for the two trainable (blue) agents, on the device."""
+class EpisodeReturns:
+    """One team's finished episodes and the sum of their returns, kept on the device the way msoc_stats keeps blue's
+    (episodes, episode_return_sum): `running` (N,) fp32 is each env's return so far in its current episode, `sums` (2,)
+    fp64 the episodes finished and their returns summed, since the last read(reset=True).  An episode that was already
+    running when counting began is counted from there."""
 
-    def __init__(self, num_steps: int, num_envs: int, device, obs_dtype=torch.float32):
-        T, N = num_steps, num_envs
-        self.obs = torch.zeros((T, N, 2, 66), dtype=obs_dtype, device=device)
-        self.actions = torch.zeros((T, N, 2, 3), device=device)
-        self.logprobs = torch.zeros((T, N, 2), device=device)
-        self.rewards = torch.zeros((T, N, 2), device=device)
-        self.dones = torch.zeros((T, N, 2), device=device)
-        self.values = torch.zeros((T, N, 2), device=device)
+    def __init__(self, num_envs: int, device):
+        self.running = torch.zeros((num_envs,), device=device)
+        self.sums = torch.zeros((2,), dtype=torch.float64, device=device)
+
+    def add(self, reward: torch.Tensor, done: torch.Tensor) -> None:
+        """One step: reward (N,) of the team, done (N,) of the same step (the truncation reward is the episode's last)."""
+        d = done.to(torch.float32)
+        self.running.add_(reward)
+        self.sums[0].add_(d.sum())
+        self.sums[1].add_((self.running * d).sum(dtype=torch.float64))
+        self.running.mul_(1.0 - d)
+
+    def read(self, reset: bool = False) -> dict:
+        out = dict(zip(("episodes", "episode_return_sum"), self.sums.tolist()))
+        if reset:
+            self.sums.zero_()
+        return out
+
+
+class RolloutBuffer:
+    """(T, N, A, ...) storage of one rollout for the A trainable agents, on the device.  agents=2: the blue agents.
+    agents=4: self-play, one policy for both teams (collect_rollout / GraphedRollout with self_play=True).  Rows 2, 3
+    are red's in the policy's frame: observations mirrored (selfplay.mirror_frames), actions as the policy returned
+    them (red played their mirror_actions), so that log-probs and PPO ratios are those of the policy; log-probs,
+    values, rewards (red's own, msoc_step_teams) and dones likewise.  `red_returns` (EpisodeReturns) then counts red's
+    finished episodes and returns over the rollouts that use this buffer; blue's are in the sim's statistics."""
+
+    def __init__(self, num_steps: int, num_envs: int, device, obs_dtype=torch.float32, agents: int = 2):
+        if agents not in (2, 4):
+            raise ValueError("agents must be 2 (blue) or 4 (both teams, self-play)")
+        T, N, A = num_steps, num_envs, agents
+        self.agents = A
+        self.obs = torch.zeros((T, N, A, 66), dtype=obs_dtype, device=device)
+        self.actions = torch.zeros((T, N, A, 3), device=device)
+        self.logprobs = torch.zeros((T, N, A), device=device)
+        self.rewards = torch.zeros((T, N, A), device=device)
+        self.dones = torch.zeros((T, N, A), device=device)
+        self.values = torch.zeros((T, N, A), device=device)
+        self.red_returns = EpisodeReturns(N, device) if A == 4 else None
 
 
 class PackedPolicy:
@@ -179,6 +213,29 @@ class PackedPolicy:
         return action, logprob, value
 
 
+def _team_rows(obs: torch.Tensor) -> torch.Tensor:
+    """(N, A, 66) rows -> (A N, 66) policy rows, team-major: [blue agents 0, 1 of every env | red agents 2, 3]."""
+    n, A = obs.shape[0], obs.shape[1]
+    if A == 2:
+        return obs.reshape(-1, 66)
+    return obs.reshape(n, 2, 2, 66).transpose(0, 1).reshape(-1, 66)
+
+
+def _per_env(x: torch.Tensor, n: int, A: int) -> torch.Tensor:
+    """Team-major policy outputs (A N, ...) -> (N, A, ...) (the inverse of _team_rows)."""
+    rest = x.shape[1:]
+    if A == 2:
+        return x.reshape(n, 2, *rest)
+    return x.reshape(2, n, 2, *rest).transpose(0, 1).reshape(n, 4, *rest)
+
+
+def _check_self_play(buf, self_play: bool, opponent) -> None:
+    if self_play and opponent is not None:
+        raise ValueError("self_play trains red with the same policy: it cannot also play an opponent")
+    if buf.obs.shape[2] != (4 if self_play else 2):
+        raise ValueError("self_play needs RolloutBuffer(agents=4); without it the buffer has 2 agents")
+
+
 def _policy_step(agent, x, policy_dtype):
     if policy_dtype is not None:
         with torch.autocast(device_type="cuda", dtype=policy_dtype):
@@ -191,41 +248,55 @@ def _policy_step(agent, x, policy_dtype):
 @torch.no_grad()
 def collect_rollout(sim, agent: Agent, normalizer: RunningMeanStd, buf: RolloutBuffer, next_obs: torch.Tensor,
                     next_done: torch.Tensor, generator=None, update_normalizer: bool = True, policy_dtype=None,
-                    deterministic: bool = False, opponent=None):
+                    deterministic: bool = False, opponent=None, self_play: bool = False):
     """One rollout of `buf.obs.shape[0]` steps (marl-soccer.ipynb:366-431): blue = policy, red = U(-1, 1), or red = the
     frozen snapshots of `opponent` (selfplay.Opponent; it samples or plays its mean as it was built to, whatever
-    `deterministic` says).  Red's observations never reach the buffer or the normaliser.
+    `deterministic` says).  Without self_play, red's observations never reach the buffer or the normaliser.
     next_obs: (N, 2, 66) raw observations of the blue agents (may be a view of the simulator's observation buffer: it is
     consumed before the next step overwrites it); next_done: (N, 2).  Returns the updated pair (next_obs is a view of
     sim.obs).  policy_dtype: optional autocast dtype for the MLPs (e.g. torch.bfloat16); the simulator is always fp32.
-    deterministic: blue plays the policy mean and red stands still (eval.py:84-104 style; used by the parity test)."""
-    T = buf.obs.shape[0]
+    deterministic: blue plays the policy mean and red stands still (eval.py:84-104 style; used by the parity test).
+    self_play: one policy plays all four agents and learns from both teams (buf = RolloutBuffer(agents=4)): red's rows
+    are mirrored into the policy's frame (selfplay.team_view), red plays mirror_actions of the policy's actions, and
+    the step is msoc_step_teams, so red gets its own reward.  next_obs is then (N, 4, 66) in the policy's frame
+    (selfplay.team_view(sim.obs)) and next_done (N, 4); the returned next_obs is a new tensor.  Red's observations
+    enter the normaliser with blue's.  With deterministic=True both teams play the policy mean."""
+    _check_self_play(buf, self_play, opponent)
+    T, A = buf.obs.shape[0], buf.obs.shape[2]
     n = sim.num_envs
     full = sim.actions  # (N, 4, 3) device buffer of the handle
     mean32, inv_std32 = normalizer.mean.float(), 1.0 / (normalizer.std.float() + 1e-8)  # fp32 on the hot loop
+    if self_play:
+        from .selfplay import mirror_actions, team_view
     for t in range(T):
         buf.obs[t] = next_obs
         buf.dones[t] = next_done
-        x = torch.clamp((next_obs.reshape(-1, 66) - mean32) * inv_std32, -10.0, 10.0)
+        x = torch.clamp((_team_rows(next_obs) - mean32) * inv_std32, -10.0, 10.0)
         if deterministic:
             action = agent.get_deterministic_action(x)
             logprob, value = torch.zeros(x.shape[0], device=x.device), agent.get_value(x)
         else:
             action, logprob, value = _policy_step(agent, x, policy_dtype)
-        buf.values[t] = value.reshape(n, 2)
-        buf.actions[t] = action.reshape(n, 2, 3)
-        buf.logprobs[t] = logprob.reshape(n, 2)
-        full[:, :2] = buf.actions[t]
-        if opponent is not None:
+        buf.values[t] = _per_env(value, n, A).reshape(n, A)
+        buf.actions[t] = _per_env(action, n, A)
+        buf.logprobs[t] = _per_env(logprob, n, A)
+        full[:, :2] = buf.actions[t, :, :2]
+        if self_play:
+            full[:, 2:] = mirror_actions(buf.actions[t, :, 2:])
+        elif opponent is not None:
             opponent.act(sim)
         elif deterministic:
             full[:, 2:] = 0.0
         else:
             full[:, 2:].uniform_(-1.0, 1.0, generator=generator)
-        obs, reward, done, _goal = sim.step(full, auto_reset=True)
+        obs, reward, done, _goal = sim.step(full, auto_reset=True, team_rewards=self_play)
         buf.rewards[t] = reward
-        next_obs = obs[:, :2]  # a view: read by the next iteration (or the caller) before the simulator steps again
-        next_done = done.to(torch.float32)[:, None].expand(n, 2)
+        if self_play:
+            buf.red_returns.add(reward[:, 2], done)
+            next_obs = team_view(obs)
+        else:
+            next_obs = obs[:, :2]  # a view: read by the next iteration (or the caller) before the simulator steps again
+        next_done = done.to(torch.float32)[:, None].expand(n, A)
     if update_normalizer:
         normalizer.update(buf.obs.reshape(-1, 66))
     return next_obs, next_done
@@ -239,22 +310,29 @@ class GraphedRollout:
     generator (graph-safe).  A sim whose states will be loaded (load_states, load_state_dict, clone_envs, set_states)
     needs one such load before the graph is captured (include/msoc.h, msoc_load_states).
     opponent: a selfplay.Opponent plays red inside the graph instead of U(-1, 1); Opponent.set() writes a new snapshot
-    into the buffers the graph reads, so the next replay plays it without a new capture."""
+    into the buffers the graph reads, so the next replay plays it without a new capture.
+    self_play: collect_rollout(self_play=True) as a graph (buf = RolloutBuffer(agents=4)): per step, blue's and red's
+    mirrored rows (msoc_team_inputs, teams 0 and 1, on the fused bf16 path; selfplay.mirror_frames otherwise) form one
+    (4N, 72) policy input, the policy runs once over it, red's actions are mirrored back into sim.actions[:, 2:] and
+    the step is msoc_step_teams.  The normaliser's moments cover both teams.  run() then returns next_obs (N, 4, 66) in
+    the policy's frame and next_done (N, 4)."""
 
     def __init__(self, sim, agent: Agent, normalizer: RunningMeanStd, buf: RolloutBuffer, policy_dtype=None,
-                 update_normalizer: bool = True, opponent=None):
+                 update_normalizer: bool = True, opponent=None, self_play: bool = False):
+        _check_self_play(buf, self_play, opponent)
         self.sim, self.agent, self.normalizer, self.buf, self.opponent = sim, agent, normalizer, buf, opponent
-        self.policy_dtype, self.update_normalizer = policy_dtype, update_normalizer
+        self.policy_dtype, self.update_normalizer, self.self_play = policy_dtype, update_normalizer, self_play
+        A = buf.obs.shape[2]
         dev = sim.device
         self.mean32 = torch.zeros((66,), device=dev)
         self.inv_std32 = torch.ones((66,), device=dev)
         self.shift32 = torch.zeros((66,), device=dev)  # -mean / (std + 1e-8)
-        self.next_done = torch.zeros((sim.num_envs, 2), device=dev)
+        self.next_done = torch.zeros((sim.num_envs, A), device=dev)
         self.graph = None
         # bf16 policy: the packed form of the two MLPs and its padded input / fp32 staging buffers
         self.packed = PackedPolicy(agent, policy_dtype) if policy_dtype is not None else None
         if self.packed is not None:
-            rows = sim.num_envs * 2
+            rows = sim.num_envs * A
             self.x32 = torch.empty((rows, 66), device=dev)
             self.x72 = torch.zeros((rows, PackedPolicy.IN), dtype=policy_dtype, device=dev)
         # per-step sums and sums of squares of the raw observations, gathered inside the graph; the running statistics merge
@@ -264,6 +342,8 @@ class GraphedRollout:
         # bf16 policy + bf16 buffer: the three consumers of the observation rows are served by one kernel of the library
         self.fused_inputs = self.packed is not None and policy_dtype == torch.bfloat16 and buf.obs.dtype == torch.bfloat16
         self._L = _capi.lib() if self.fused_inputs else None
+        if self.fused_inputs and self_play:  # the raw rows of the two teams, team-major, before they go to the buffer
+            self.raw2 = torch.zeros((2, sim.num_envs, 2, 66), dtype=buf.obs.dtype, device=dev)
 
     def _refresh(self):
         self.mean32.copy_(self.normalizer.mean.float())
@@ -274,6 +354,8 @@ class GraphedRollout:
 
     @torch.no_grad()
     def _body(self):
+        if self.self_play:
+            return self._body_self_play()
         sim, buf, n = self.sim, self.buf, self.sim.num_envs
         full = sim.actions
         self.moments.zero_()
@@ -314,6 +396,51 @@ class GraphedRollout:
             buf.rewards[t] = reward
             self.next_done.copy_(done.to(torch.float32)[:, None].expand(n, 2))
 
+    def _body_self_play(self):
+        from .selfplay import mirror_actions, mirror_frames
+        sim, buf, n = self.sim, self.buf, self.sim.num_envs
+        full = sim.actions
+        stream = torch.cuda.current_stream(sim.device).cuda_stream
+        self.moments.zero_()
+        for t in range(buf.obs.shape[0]):
+            buf.dones[t] = self.next_done
+            if self.fused_inputs:
+                # one pass per team (msoc_team_inputs; team 1 mirrors red's rows): rows [0, 2N) of the policy input are
+                # blue's, [2N, 4N) red's; raw rows to the buffer; moments of both teams into the same sums
+                for team in (0, 1):
+                    _capi.check(self._L.msoc_team_inputs(sim.obs.data_ptr(), n, team, self.shift32.data_ptr(),
+                                                         self.inv_std32.data_ptr(), self.x72[2 * n * team:].data_ptr(),
+                                                         self.raw2[team].data_ptr(),
+                                                         self.moments[t].data_ptr() if self.update_normalizer else None,
+                                                         stream))
+                buf.obs[t].view(n, 2, 2, 66).copy_(self.raw2.transpose(0, 1))
+            else:
+                rows = torch.cat([sim.obs[:, :2], mirror_frames(sim.obs[:, 2:])], 1)  # (N, 4, 66), the policy's frame
+                buf.obs[t] = rows
+                x = _team_rows(rows)
+                if self.update_normalizer:
+                    v, m = torch.var_mean(x, dim=0, unbiased=False)
+                    self.moments[t, 0].copy_(m * (4 * n))
+                    self.moments[t, 1].copy_((v + m.square()) * (4 * n))
+                if self.packed is not None:
+                    torch.addcmul(self.shift32, x, self.inv_std32, out=self.x32)
+                    self.x32.clamp_(-10.0, 10.0)
+                    self.x72[:, :66].copy_(self.x32)
+            if self.packed is not None:
+                action, logprob, value = self.packed.act(self.x72)
+            else:
+                x = torch.clamp((x - self.mean32) * self.inv_std32, -10.0, 10.0)
+                action, logprob, value = _policy_step(self.agent, x, self.policy_dtype)
+            buf.values[t] = _per_env(value, n, 4).reshape(n, 4)
+            buf.actions[t] = _per_env(action, n, 4)
+            buf.logprobs[t] = _per_env(logprob, n, 4)
+            full[:, :2] = buf.actions[t, :, :2]
+            full[:, 2:] = mirror_actions(buf.actions[t, :, 2:])
+            _obs, reward, done, _goal = sim.step(full, auto_reset=True, team_rewards=True)
+            buf.rewards[t] = reward
+            buf.red_returns.add(reward[:, 2], done)
+            self.next_done.copy_(done.to(torch.float32)[:, None].expand(n, 4))
+
     def run(self):
         """One rollout; returns (next_obs view, next_done)."""
         self._refresh()
@@ -331,21 +458,25 @@ class GraphedRollout:
         else:
             self.graph.replay()
         if self.update_normalizer:
-            count = self.moments.shape[0] * self.sim.num_envs * 2
+            count = self.moments.shape[0] * self.sim.num_envs * self.buf.obs.shape[2]
             total = self.moments.sum(0)
             mean = total[0] / count
             self.normalizer.update_from_moments(mean, total[1] / count - mean.square(), count)
+        if self.self_play:
+            from .selfplay import team_view
+            return team_view(self.sim.obs), self.next_done
         return self.sim.obs[:, :2], self.next_done
 
 
 @torch.no_grad()
 def compute_gae(agent: Agent, normalizer: RunningMeanStd, buf: RolloutBuffer, next_obs, next_done, gamma=0.995,
                 gae_lambda=0.95):
-    """Generalised advantage estimation over the rollout (marl-soccer.ipynb:454-464)."""
-    T, n = buf.rewards.shape[0], buf.rewards.shape[1]
-    next_value = agent.get_value(normalizer.normalize(next_obs.reshape(-1, 66))).reshape(n, 2)
+    """Generalised advantage estimation over the rollout (marl-soccer.ipynb:454-464), for any number of agents A per env
+    (buf.rewards (T, N, A); next_obs (N, A, 66), next_done (N, A))."""
+    T, n, A = buf.rewards.shape
+    next_value = agent.get_value(normalizer.normalize(next_obs.reshape(-1, 66))).reshape(n, A)
     adv = torch.zeros_like(buf.rewards)
-    last = torch.zeros((n, 2), device=buf.rewards.device)
+    last = torch.zeros((n, A), device=buf.rewards.device)
     for t in reversed(range(T)):
         nonterminal = 1.0 - (next_done if t == T - 1 else buf.dones[t + 1])
         nv = next_value if t == T - 1 else buf.values[t + 1]

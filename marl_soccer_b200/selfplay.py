@@ -5,7 +5,9 @@ msoc_team_inputs), so a blue policy plays red unchanged when it sees red's frame
 back.  `mirror_frames` / `mirror_actions` are that transform (the reference implementation the CUDA kernel is tested
 against, and the helpers for host users of SyncMultiAgentVecEnv / HostBufferSim who run their own red policy).
 `Opponent` is a pool of frozen snapshots playing red in contiguous slices of the envs, inside collect_rollout /
-GraphedRollout (rollout.py) or `evaluate_match`.  Red gets no reward: only blue learns.
+GraphedRollout (rollout.py) or `evaluate_match`; red then gets no reward and only blue learns.  For one policy that
+learns from both teams, collect_rollout / GraphedRollout take self_play=True instead (msoc_step_teams gives red its own
+reward; `team_view` is the observation that policy sees).
 """
 from __future__ import annotations
 
@@ -41,6 +43,14 @@ def mirror_frames(x):
     for s in _NEG_SLICES:
         f[..., s] = -f[..., s]
     return f.reshape(x.shape)
+
+
+def team_view(obs):
+    """(N, 4, 66) observation rows -> the same rows in the frame of a policy that plays both teams (self-play): blue's
+    rows 0, 1 as they are, red's rows 2, 3 mirrored (mirror_frames).  A new tensor or array."""
+    if isinstance(obs, np.ndarray):
+        return np.concatenate([obs[:, :2], mirror_frames(obs[:, 2:])], 1)
+    return torch.cat([obs[:, :2], mirror_frames(obs[:, 2:])], 1)
 
 
 def mirror_actions(a):

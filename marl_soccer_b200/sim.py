@@ -45,6 +45,7 @@ class BatchedSoccerSim:
     step() returns views of internal buffers that stay valid until the next step():
       obs    (N, 4, 66) float32   3 stacked 22-float frames per agent, newest last (soccer_env.py:37-39)
       reward (N, 2)     float32   blue agents only; red is always 0.0 (soccer_env.py:141-146)
+                (N, 4)     float32   with step(..., team_rewards=True): blue's in columns 0, 1, red's own reward in 2, 3
       done   (N,)       uint8     truncation at max_steps (soccer_env.py:148); never "terminated"
       goal   (N,)       int8      +1 blue scored, -1 red scored (info["goal_scored_by"])
       score  (N, 2)     int32     info["score"] of the step, before any auto-reset
@@ -80,6 +81,7 @@ class BatchedSoccerSim:
         self.score = _view(bufs.score, (n, 2), "<i4", d)
         self._stats = torch.zeros((8,), dtype=torch.float64, device=d)
         self._stats_live = _view(bufs.stats, (8,), "<f8", d)  # the accumulators themselves (state_dict)
+        self.reward4 = None  # (N, 4) rewards of step(team_rewards=True), allocated by its first call
 
     def _index(self, idx, unique: bool = False, n_all: int | None = None):
         """(int64 CUDA tensor or None, count) of an env index argument: None (envs 0..n_all-1, default all), a host
@@ -124,19 +126,31 @@ class BatchedSoccerSim:
                                        self._stream()))
         return self.obs
 
-    def step(self, actions: torch.Tensor, auto_reset: bool = True, general_path: bool = False):
+    def step(self, actions: torch.Tensor, auto_reset: bool = True, general_path: bool = False, team_rewards: bool = False):
         """One env-step for every env.  actions: (N, 4, 3) float32 CUDA tensor in [-1, 1] (clipped on
         the device like soccer_env.py:119).  general_path (debugging / tests): every env that touches something is
-        stepped by the general contact path instead of its work class's own."""
+        stepped by the general contact path instead of its work class's own.
+        team_rewards: step with msoc_step_teams; the reward returned is then `self.reward4` (N, 4): blue's reward
+        in columns 0, 1 (what the plain step returns), red's own reward in 2, 3 (include/msoc.h).  That tensor is
+        allocated by the first such call, which therefore must not be inside a CUDA graph capture."""
         if actions.device != self.device or actions.dtype != torch.float32 or not actions.is_contiguous():
             actions = actions.to(device=self.device, dtype=torch.float32).contiguous()
         if actions.numel() != self.num_envs * 12:
             raise ValueError(f"actions must have shape ({self.num_envs}, 4, 3), got {tuple(actions.shape)}")
+        flags = (_capi.STEP_AUTO_RESET if auto_reset else 0) | (_capi.STEP_GENERAL_PATH if general_path else 0)
+        if team_rewards:
+            if self.reward4 is None:
+                if torch.cuda.is_current_stream_capturing():
+                    raise RuntimeError("the first step(team_rewards=True) allocates the (N, 4) reward tensor: "
+                                       "call it once before capturing a CUDA graph")
+                self.reward4 = torch.zeros((self.num_envs, 4), dtype=torch.float32, device=self.device)
+            _capi.check(self._L.msoc_step_teams(self._h, actions.data_ptr(), self.obs.data_ptr(),
+                                                self.reward4.data_ptr(), self.done.data_ptr(), self.goal.data_ptr(),
+                                                self.score.data_ptr(), flags, self._stream()))
+            return self.obs, self.reward4, self.done, self.goal
         _capi.check(self._L.msoc_step(self._h, actions.data_ptr(), self.obs.data_ptr(),
                                       self.reward.data_ptr(), self.done.data_ptr(), self.goal.data_ptr(),
-                                      self.score.data_ptr(),
-                                      (_capi.STEP_AUTO_RESET if auto_reset else 0) | (_capi.STEP_GENERAL_PATH if general_path else 0),
-                                      self._stream()))
+                                      self.score.data_ptr(), flags, self._stream()))
         return self.obs, self.reward, self.done, self.goal
 
     def stats_tensor(self, reset: bool = False) -> torch.Tensor:
