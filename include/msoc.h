@@ -185,7 +185,9 @@ int msoc_step_teams(msoc_handle *h, const float *d_actions, float *d_obs_out,
 /* Same call with HOST buffers (the NumPy drop-in path, marl_vecenv.py:62-68): copies actions
    H2D, steps, copies obs/reward/done/goal D2H and synchronises; NULL output pointers are skipped.  Large batches are
    cut into up to 8 chunks on two internal streams so that the H2D copy and the kernels of one chunk overlap the D2H
-   copies of the previous one.  Pinned host memory is used as given. */
+   copies of the previous one.  Pinned host memory is used as given.  Host-buffer steps, device steps (msoc_step,
+   msoc_step_teams), replays of captured graphs of them, resets and state loads may be interleaved on one handle in any
+   order: each step continues from the state the previous call left. */
 int msoc_step_host(msoc_handle *h, const float *h_actions, float *h_obs, float *h_reward,
                    uint8_t *h_done, int8_t *h_goal, int32_t *h_score, uint32_t flags, void *stream);
 /* The same step, but only the NEWEST frame comes back: h_frames (N,4,22) f32 = 352 B per env instead of 1 056.  The

@@ -1287,6 +1287,10 @@ static int step_host_impl(msoc_handle *h, const float *h_actions, float *h_obs, 
         return MSOC_OK;
     }
     CUDA_TRY(cudaMemsetAsync(h->d_ctl + CTL_CHUNK0, 0, CTL_WORDS * MAX_CHUNKS * sizeof(int), st));
+    /* A whole step expects the list counters of its parity to be zero: the streaming kernel of the previous whole step
+       clears them, and the chunks of this step do not.  Clear both sets, so that a device step or a graph replay may
+       follow on the same handle.  (Words 16.. hold the step counters and the last class counts.) */
+    CUDA_TRY(cudaMemsetAsync(h->d_ctl, 0, 2 * CTL_WORDS * sizeof(int), st));
     CUDA_TRY(cudaEventRecord(h->ev_pipe_fork, st));
     CUDA_TRY(cudaStreamWaitEvent(h->pipe_stream, h->ev_pipe_fork, 0));
     for (int c = 0; c < chunks; c++) {
